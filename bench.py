@@ -4,9 +4,9 @@
 
   python bench.py --gpus N --steps K --warmup W            our CUDA path
   python bench.py --impl reference ...                     the reference's own CPU implementation on the host cores:
-                                                           the UNMODIFIED reference modules (baseline/_ref, a git-ignored
-                                                           copy made by __graft_entry__.build(), run under oracle/ref_shims)
-                                                           or, if that copy is absent, the oracle port
+                                                           the UNMODIFIED reference modules (oracle/_ref, a git-ignored
+                                                           copy made by __graft_entry__.build(), or GIMS_REFERENCE_ROOT;
+                                                           run under oracle/ref_shims) or, if absent, the oracle port
   --kpts N                                                 keypoints per image (BASELINE configs[3] = 4096, configs[4] = 8192)
   --weights random|damped                                  random-init weights (degenerate scores: mean 0.3, std 0.002) or
                                                            the non-degenerate "damped" set (scores ~ 90 +- 2.6 like a trained net)
@@ -18,6 +18,8 @@ A step = one batch of `--pairs-per-step` synthetic pairs per GPU through the who
             `--e2e-threads` host threads with one CUDA stream each; `single_thread_value` = one caller.
 `roofline`: dominant kernel, timed live with CUDA events inside the library on its own stream.
 Multi-GPU: one process per GPU (torchrun), pairs sharded, no collective on the data path (weak scaling).
+`--dump-outputs DIR` writes what the last timed step returned (see `dump_outputs`) so that two builds can be compared
+output for output: the inputs depend only on the arguments.
 """
 import argparse
 import json
@@ -37,6 +39,7 @@ from gims_b200.synth import make_pair, make_state_dict  # noqa: E402
 
 UNIT = 'pairs/s'
 FALLBACK_PEAKS = {'hbm_gbs': 6650.0, 'bf16_tflops': 1590.0, 'bf16_tflops_sustained': 1400.0}
+DUMP_LIMIT_BYTES = 64 * 10 ** 6           # --dump-outputs, all files
 
 
 def metric_name(kpts):
@@ -213,6 +216,30 @@ class ClockSampler:
         return {'sm_mhz': med, 'sm_max_mhz': smax, 'reasons': sorted(reasons), 'samples': len(sm), 'source': 'nvidia-smi'}
 
 
+def dump_outputs(path, outs, kpts):
+    """Write what one step of `PairBatchRunner.run` returned to its caller, pairs in step order, as `path/<name>.npy`:
+      counts.npy            (P, 8) float64  the library's per-pair counters: N' of both images, edges, components, status
+      matches0.npy          (sum of N'0,) float64  per pair, for each kept keypoint of image 0: the index of its match
+                            among the kept keypoints of image 1, or -1; pairs one after the other (counts[:, 0] splits them)
+      matching_scores0.npy  (sum of N'0,) float32  laid out like matches0
+      pair_index.npy        (P,) float64  position of each pair in the step
+    When the pairs could exceed DUMP_LIMIT_BYTES, a fixed seeded sample of them is written instead."""
+    import numpy as np
+    per_pair = 9 * 8 + kpts * (8 + 4)                  # N'0 <= kpts
+    room = DUMP_LIMIT_BYTES - 4 * 128                   # .npy headers
+    idx = np.arange(len(outs))
+    if len(outs) * per_pair > room:
+        idx = np.sort(np.random.default_rng(0).choice(len(outs), room // per_pair, replace=False))
+    counts = np.stack([outs[i]['n_kept_dev'].cpu().numpy() for i in idx]).astype(np.float64)
+    kept = [int(c) for c in counts[:, 0]]
+    matches = np.concatenate([outs[i]['matches0'][:n].cpu().numpy() for i, n in zip(idx, kept)]).astype(np.float64)
+    scores = np.concatenate([outs[i]['mscores0'][:n].cpu().numpy() for i, n in zip(idx, kept)]).astype(np.float32)
+    os.makedirs(path, exist_ok=True)
+    for name, arr in (('counts', counts), ('matches0', matches), ('matching_scores0', scores),
+                      ('pair_index', idx.astype(np.float64))):
+        np.save(os.path.join(path, name + '.npy'), arr)
+
+
 def measure_tf32_peak(dev):
     """Dense TF32 tensor throughput of this GPU (cuBLAS, 8192^3), measured like MEASURED_PEAKS.json's bf16 number
     (SURVEY.md 8d asks for it: the file has no TF32 entry).  Used only as a roofline denominator."""
@@ -238,18 +265,15 @@ def measure_tf32_peak(dev):
 
 def _reference_runner(args):
     """Callable one(seed) that runs one pair of the bench workload through the reference's CPU implementation, and
-    a description of what it is.  Preferred: the unmodified reference modules copied to baseline/_ref (git-ignored,
-    made by __graft_entry__.build() where /root/reference exists; they travel to the GPU box) imported under
+    a description of what it is.  Preferred: the unmodified reference modules (ref_shims.REFERENCE_ROOT: the
+    git-ignored copy in oracle/_ref made by __graft_entry__.build(), or GIMS_REFERENCE_ROOT) imported under
     oracle/ref_shims.py.  Fallback: the oracle port."""
     import contextlib
     import io
     sd = make_state_dict(0, damped=(args.weights == 'damped'))
     cfg = {'sinkhorn_iterations': 100, 'match_threshold': 0.2}
-    ref_root = os.path.join(ROOT, 'baseline', '_ref')
-    if os.path.isfile(os.path.join(ref_root, 'models', 'gmatcher.py')) and not os.environ.get('GIMS_BENCH_FORCE_PORT'):
-        os.environ['GIMS_REFERENCE_ROOT'] = ref_root
-        from oracle import ref_shims
-        ref_shims.REFERENCE_ROOT = ref_root
+    from oracle import ref_shims
+    if ref_shims.reference_available() and not os.environ.get('GIMS_BENCH_FORCE_PORT'):
         _, gm = ref_shims.load_reference()
         model = gm.GMatcher(cfg)
         model.load_state_dict(sd)
@@ -260,7 +284,7 @@ def _reference_runner(args):
             data.update({'radius': 25, 'percentile': 7, 'min_size': 8, 'device': torch.device('cpu')})
             with torch.no_grad(), contextlib.redirect_stdout(io.StringIO()):
                 return model(data)
-        return one, 'reference', 'unmodified reference models/{agc,gmatcher}.py (baseline/_ref) under oracle/ref_shims.py'
+        return one, 'reference', 'unmodified reference models/{agc,gmatcher}.py under oracle/ref_shims.py'
     from oracle import gims_oracle as orc
 
     def one(seed):
@@ -278,10 +302,9 @@ def run_reference(args, rank, world):
     cores = os.cpu_count() or 1
     torch.set_num_threads(cores)
     one, kind, what = _reference_runner(args)
-    # bounded sample: each step is one pair; cap the run at a few minutes whatever --steps says
-    per_pair_guess = {2048: 1.5, 4096: 8.0, 8192: 45.0}.get(args.kpts, 1.5 * (args.kpts / 2048.0) ** 2.3)
-    steps = max(1, min(args.steps, int(180.0 / per_pair_guess)))
-    for w in range(1 if per_pair_guess < 20 else 0):
+    # each step is one pair on the host (seconds at 2048 keypoints, most of a minute at 8192)
+    steps = args.steps
+    for w in range(args.warmup):
         one(1000 + w)
     t0 = time.perf_counter()
     for s in range(steps):
@@ -294,8 +317,7 @@ def run_reference(args, rank, world):
         'scaling': 'weak', 'vs_baseline': None, 'dtype': 'f32', 'data': 'synthetic',
         'config': base_config(args, world),
         'cpu_baseline': {'value': val, 'unit': UNIT, 'cores': cores, 'kind': kind,
-                         'sample': 'one pair per step, %d steps timed (bounded sample of the same workload), %s, torch %d '
-                                   'threads' % (steps, what, cores)},
+                         'sample': 'one pair per step, %d steps timed, %s, torch %d threads' % (steps, what, cores)},
         'e2e': {'value': val, 'unit': UNIT, 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0},
         'gpu_launches': 0,
     }
@@ -320,9 +342,10 @@ def cpu_baseline(args):
 
 def load_caller_carhynet(dev):
     """The CALLER's descriptor object of the pipeline config: the reference's CAR_HyNet (random init — the trained
-    weights are not in the reference tree) from the git-ignored copy under baseline/_ref, wrapped like
+    weights are not in the reference tree) from the reference under oracle/ref_shims.py's REFERENCE_ROOT, wrapped like
     carhynet/models.py:639-670 `HyNetnetFeature2D` (whose __init__ hard-loads ./weights/car_hynet.pth)."""
-    ref_root = os.path.join(ROOT, 'baseline', '_ref')
+    from oracle import ref_shims
+    ref_root = ref_shims.REFERENCE_ROOT
     if not os.path.isfile(os.path.join(ref_root, 'carhynet', 'models.py')):
         return None
     if ref_root not in sys.path:
@@ -345,14 +368,14 @@ def run_pipeline(args):
     torch.cuda.set_device(dev)
     car = load_caller_carhynet(dev)
     if car is None:
-        print(json.dumps({'metric': 'pipeline_pairs_per_sec_800x600', 'unavailable': 'baseline/_ref/carhynet is missing '
-                          '(run __graft_entry__.build() where /root/reference exists)'}))
+        print(json.dumps({'metric': 'pipeline_pairs_per_sec_800x600', 'unavailable': 'the reference\'s carhynet/ is missing '
+                          '(run __graft_entry__.build() with GIMS_REFERENCE_ROOT set to a reference checkout)'}))
         return
     max_kp = args.kpts
     matching = Matching({'sinkhorn_iterations': 20, 'match_threshold': 0.2, 'max_keypoints': max_kp})
     matching.gmodel.load_state_dict(make_state_dict(0, damped=(args.weights == 'damped')))
     matching = matching.eval().to(dev)
-    n_pairs = max(3, args.steps)
+    n_pairs = args.steps
     pairs = []
     for i in range(n_pairs + 1):
         img0 = make_textured_image(600, 800, seed=100 + i)
@@ -444,7 +467,13 @@ def main():
     ap.add_argument('--pipeline', action='store_true',
                     help='BASELINE configs[2]: eval_homography-shaped pipeline (synthetic 800x600 image pairs -> SIFT + '
                          'patches on the host -> CAR-HyNet on the GPU -> matcher), the literal call of eval_homography.py:177')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last one computed as DIR/<name>.npy (see dump_outputs)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.pipeline or args.impl != 'ours'):
+        ap.error('--dump-outputs writes the outputs of the CUDA path (--impl ours, without --pipeline)')
     if args.pipeline:
         run_pipeline(args)
         return
@@ -522,6 +551,8 @@ def main():
     ms = e0.elapsed_time(e1)
     launches = L.gims_launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, outs, args.kpts)
     if world > 1:
         t = torch.tensor([ms], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

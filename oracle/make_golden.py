@@ -1,6 +1,6 @@
 """TEST INFRASTRUCTURE — generate `tests/golden/*.npz` by running the UNMODIFIED reference.
 
-Run in the build container only (needs /root/reference):   python -m oracle.make_golden
+Needs a checkout of the reference:   GIMS_REFERENCE_ROOT=<songxf1024/GIMS checkout> python -m oracle.make_golden
 Each fixture holds the synthetic-input recipe (sizes, seed, knobs — inputs are regenerated from
 `gims_b200.synth`, not stored) and the reference's outputs at that boundary:
   * graph fixtures (`agc_*.npz`): kept indices + relabelled CSR per image, from

@@ -1,12 +1,12 @@
 """TEST INFRASTRUCTURE — import shims that let the UNMODIFIED reference run in this container.
 
 Only `oracle/make_golden.py`, `tests/test_oracle_vs_reference.py` and the reference arm of `bench.py`
-(`--impl reference`, on the git-ignored copy under baseline/_ref) use this file.  It never travels into the
+(`--impl reference`) use this file, on the reference named by REFERENCE_ROOT below.  It never travels into the
 product path.
 
 The reference imports three packages that are absent here (SURVEY.md Appendix A):
 `matplotlib` (import only), `torch_scatter` (training loss only) and `dgl` — pinned `dgl==1.1.2+cu117`
-in /root/reference/requirements:16, not vendored.  The dgl surface the hot path touches is restated
+in the reference's requirements:16, not vendored.  The dgl surface the hot path touches is restated
 from DGL's published semantics:
 
 * `dgl.from_networkx(g, device=)` (python/dgl/convert.py): nodes relabelled with
@@ -25,7 +25,9 @@ import os
 import sys
 import types
 
-REFERENCE_ROOT = os.environ.get('GIMS_REFERENCE_ROOT', '/root/reference')
+# a checkout of songxf1024/GIMS named by GIMS_REFERENCE_ROOT, else the copy of its modules that
+# __graft_entry__.install_reference() leaves in the git-ignored oracle/_ref; the repository itself does not contain it
+REFERENCE_ROOT = os.environ.get('GIMS_REFERENCE_ROOT') or os.path.join(os.path.dirname(os.path.abspath(__file__)), '_ref')
 
 
 def reference_available():
@@ -125,12 +127,12 @@ _REF = None
 
 
 def load_reference():
-    """Import /root/reference/models/{agc,gmatcher}.py unchanged; returns (agc_module, gmatcher_module)."""
+    """Import models/{agc,gmatcher}.py of REFERENCE_ROOT unchanged; returns (agc_module, gmatcher_module)."""
     global _REF
     if _REF is not None:
         return _REF
     if not reference_available():
-        raise RuntimeError('reference tree not present at %s' % REFERENCE_ROOT)
+        raise RuntimeError('reference tree not present at %s (set GIMS_REFERENCE_ROOT)' % REFERENCE_ROOT)
     _install_stubs()
     if REFERENCE_ROOT not in sys.path:
         sys.path.insert(0, REFERENCE_ROOT)

@@ -1,5 +1,7 @@
-"""CPU, build container only: gims_b200.frontend.sift_forward against the UNMODIFIED reference `sift_forward`
-(utils/common.py:837-893) with the reference's own CAR_HyNet (random init) on a synthetic textured image."""
+"""CPU: gims_b200.frontend.sift_forward against the UNMODIFIED reference `sift_forward` (utils/common.py:837-893) with
+the reference's own CAR_HyNet (random init) on a synthetic textured image.  The reference is not part of the repository:
+these tests run where it is installed (oracle/_ref, copied by __graft_entry__.build() from GIMS_REFERENCE_ROOT, or
+GIMS_REFERENCE_ROOT itself)."""
 import contextlib
 import io
 import sys
@@ -11,7 +13,7 @@ import torch
 from oracle.ref_shims import REFERENCE_ROOT, _install_stubs, reference_available
 
 cv2 = pytest.importorskip('cv2')
-pytestmark = pytest.mark.skipif(not reference_available(), reason='reference tree not present')
+pytestmark = pytest.mark.skipif(not reference_available(), reason='needs the original GIMS code (oracle/_ref or GIMS_REFERENCE_ROOT)')
 
 
 def _textured(h, w, seed, color=True):

@@ -546,21 +546,32 @@ def test_bf16_variant_report(name):
     assert agree_idx >= 0.9 and agree_m >= 0.9
 
 
+class _PatchNet(torch.nn.Module):
+    """Stands in for the caller's CAR-HyNet (whose definition lives in the reference, not here): colour 32x32 patches ->
+    unit-norm 128-d descriptors, random init.  The front-end treats the caller's network as opaque."""
+
+    def __init__(self):
+        super().__init__()
+        self.body = torch.nn.Sequential(torch.nn.Conv2d(3, 32, 3, stride=2, padding=1), torch.nn.ReLU(),
+                                        torch.nn.Conv2d(32, 64, 3, stride=2, padding=1), torch.nn.ReLU(),
+                                        torch.nn.Conv2d(64, 128, 8))
+
+    def forward(self, x):
+        return torch.nn.functional.normalize(self.body(x).flatten(1), dim=1)
+
+
 def test_eval_homography_literal_call():
-    """§8f row 1: the call every script of the reference makes (eval_homography.py:177) — images + the caller's CAR-HyNet,
-    no keypoints — against the same call with the front-end run by hand and fed in as keypoints / descriptors."""
-    import os
-    import sys
+    """§8f row 1: the call every script of the reference makes (eval_homography.py:177) — images + the caller's descriptor
+    network, no keypoints — against the same call with the front-end run by hand and fed in as keypoints / descriptors.
+    The network is `_PatchNet`, a stand-in, not the reference's CAR-HyNet: both calls run the same network, which is all
+    the comparison needs."""
+    import types
     pytest.importorskip('cv2')
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    if not os.path.isfile(os.path.join(root, 'baseline', '_ref', 'carhynet', 'models.py')):
-        pytest.skip('baseline/_ref/carhynet missing (made by __graft_entry__.build() where /root/reference exists)')
-    sys.path.insert(0, root)
-    from bench import load_caller_carhynet
     from gims_b200 import Matching, frontend
     from gims_b200.synth import make_textured_image, warp_image
     dev = torch.device('cuda')
-    car = load_caller_carhynet(dev)
+    torch.manual_seed(0)
+    car = types.SimpleNamespace(model=_PatchNet().to(dev).eval(), batch_size=512)   # the wrapper's fields describe() reads
     matching = Matching({'sinkhorn_iterations': 20, 'match_threshold': 0.01, 'max_keypoints': 700})
     matching.gmodel.load_state_dict(make_state_dict(0, damped=True))
     matching = matching.eval().to(dev)

@@ -1,5 +1,6 @@
-"""CPU, build container only: the oracle restatement against the UNMODIFIED reference run live (oracle/ref_shims.py),
-on inputs that are not among the committed fixtures.  Skipped where /root/reference does not exist (the GPU box)."""
+"""CPU: the oracle restatement against the UNMODIFIED reference run live (oracle/ref_shims.py), on inputs that are not
+among the committed fixtures.  The reference is not part of the repository: these tests run where it is installed
+(oracle/_ref, copied by __graft_entry__.build() from GIMS_REFERENCE_ROOT, or GIMS_REFERENCE_ROOT itself)."""
 import contextlib
 import io
 
@@ -9,9 +10,9 @@ import torch
 
 from gims_b200.synth import make_pair, make_state_dict
 from oracle import gims_oracle as orc
-from oracle.ref_shims import load_reference, reference_available
+from oracle.ref_shims import REFERENCE_ROOT, load_reference, reference_available
 
-pytestmark = pytest.mark.skipif(not reference_available(), reason='reference tree not present')
+pytestmark = pytest.mark.skipif(not reference_available(), reason='needs the original GIMS code (oracle/_ref or GIMS_REFERENCE_ROOT)')
 
 
 @pytest.mark.parametrize('n0,n1,seed,r,p,m', [(260, 231, 901, 25, 7, 8), (400, 400, 902, 15, 2, 7), (150, 90, 903, 30, 20, 3)])
@@ -58,7 +59,7 @@ def test_gt_matches_equal_live_reference():
     import importlib
     import sys
     load_reference()
-    sys.path.insert(0, '/root/reference')
+    sys.path.insert(0, REFERENCE_ROOT)
     try:
         with contextlib.redirect_stdout(io.StringIO()):
             pu = importlib.import_module('utils.preprocess_utils')
