@@ -131,6 +131,11 @@ SIGNATURES = {
     'gims_extract_patches': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p,
                                        C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     'gims_debug_bicubic_table': (C.c_int, [C.c_void_p]),
+    'gims_pyramid_layout': (C.c_int, [C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), C.c_void_p, C.c_void_p, C.c_void_p]),
+    'gims_pyramid_workspace_bytes': (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
+    'gims_gaussian_pyramid': (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_size_t,
+                                        C.c_void_p]),
+    'gims_debug_gaussian_kernel': (C.c_int, [C.c_double, C.c_void_p, C.POINTER(C.c_int)]),
     'gims_gt_workspace_bytes': (C.c_size_t, [C.c_int, C.c_int]),
     'gims_gt_matches': (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_float, C.c_int, C.c_void_p,
                                   C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -1,7 +1,7 @@
 // Oriented keypoint patches on the device (SURVEY.md §8f row 2): replaces the per-keypoint loop of `ComputePatches`
 // (utils/library.py:84-110: cv2.warpAffine(level, M, (64, 64), INTER_CUBIC, BORDER_CONSTANT) for every keypoint) and the
-// 64 -> 32 px INTER_AREA resize + /255 of utils/common.py:882-884.  The Gaussian pyramid itself stays with OpenCV on the
-// host (23 ms per image; the loop this kernel replaces is 200-500 ms per image).
+// 64 -> 32 px INTER_AREA resize + /255 of utils/common.py:882-884.  The Gaussian pyramid it reads is built by
+// pyramid.cu, or by OpenCV on the host and uploaded (the loop this kernel replaces is 200-500 ms per image).
 //
 // The patch must be what OpenCV produces, bit for bit — the descriptors and therefore the matches depend on it — so the
 // kernel follows OpenCV's 8-bit fixed-point warp exactly (imgproc/src/imgwarp.cpp, WarpAffineInvoker + remapBicubic):

@@ -8,7 +8,8 @@ Mirrors `sift_forward` (utils/common.py:837-893): OpenCV SIFT detection, OpenCV-
 128-d descriptor duplicated to 256-d (utils/common.py:891).
 
 What is different from the reference, and why:
-  * detection and the Gaussian pyramid stay on the host (OpenCV); the per-keypoint patch loop (§8f row 2: cv2.warpAffine
+  * detection stays on the host (OpenCV); the Gaussian pyramid of a uint8 grey or colour image is built on the device,
+    byte for byte what OpenCV builds (`gaussian_pyramid_device`, csrc/pyramid.cu), while the host detects; the per-keypoint patch loop (§8f row 2: cv2.warpAffine
     + resize per keypoint, 200-500 ms per image) runs as ONE kernel on the device that reproduces OpenCV's fixed-point
     cubic warp bit for bit (`extract_patches_device`, csrc/patches.cu; GIMS_HOST_PATCHES=1 keeps the host loop);
   * the descriptor network runs on the device the matcher lives on and its output NEVER leaves it: the reference
@@ -174,21 +175,133 @@ def _pinned_staging(nbytes):
     return buf
 
 
+class DevicePyramid:
+    """The Gaussian pyramid of one image on the device (`gaussian_pyramid_device`): every level in one uint8 buffer and
+    the level table `gims_extract_patches` reads.  `buffer` uint8, `offset` int64, `height` / `width` int32 are device
+    tensors; `shapes` is the host copy of the level sizes."""
+
+    def __init__(self, buffer, offset, height, width, shapes, offsets, channels):
+        self.buffer, self.offset, self.height, self.width = buffer, offset, height, width
+        self.shapes, self.offsets, self.channels = shapes, offsets, channels
+
+    def __len__(self):
+        return len(self.shapes)
+
+    def level(self, i):
+        """Level i as a (H, W[, C]) uint8 device tensor (a view of the buffer); the same shape as the host level."""
+        h, w = self.shapes[i]
+        o = int(self.offsets[i])
+        v = self.buffer[o:o + h * w * self.channels]
+        return v.view(h, w, self.channels) if self.channels == 3 else v.view(h, w)
+
+
+_PYR_WS = {}                    # (device, stream, thread) -> grow-only uint8 workspace of gims_gaussian_pyramid
+_PYR_WS_LOCK = __import__('threading').Lock()
+
+
+def pyramid_on_device(image):
+    """True if `gaussian_pyramid_device` can build this image's pyramid: uint8, grey or 3-channel colour."""
+    a = np.asarray(image)
+    return a.dtype == np.uint8 and (a.ndim == 2 or (a.ndim == 3 and a.shape[2] in (1, 3))) and a.size > 0
+
+
+def gaussian_pyramid_device(image, device):
+    """`gaussian_pyramid` on the GPU, byte for byte the same levels (csrc/pyramid.cu follows OpenCV's 8-bit fixed-point
+    resize and blur).  Only the image travels: it is copied through the calling thread's pinned staging buffer and the
+    pyramid is enqueued on the current stream of `device`; nothing waits for it.  Returns a `DevicePyramid`, which
+    `extract_patches_device` takes in place of host levels.  The level buffer belongs to the returned object (the
+    pyramids of several images may be alive at once); the row-pass workspace is cached per (device, stream, thread),
+    grow-only, and its reuse is ordered by the stream."""
+    import ctypes as C
+    from . import _lib
+    dev = torch.device(device)
+    if dev.type != 'cuda':
+        raise _lib.GimsError('gaussian_pyramid_device needs a CUDA device')
+    img = np.asarray(image)
+    if not pyramid_on_device(img):
+        raise _lib.GimsError('gaussian_pyramid_device: need a uint8 (H, W), (H, W, 1) or (H, W, 3) image (got %s %s)'
+                             % (img.dtype, img.shape))
+    h, w = img.shape[:2]
+    cn = 3 if img.ndim == 3 and img.shape[2] == 3 else 1
+    L = _lib.lib()
+    n = C.c_int(0)
+    _lib.check(L.gims_pyramid_layout(h, w, cn, C.byref(n), None, None, None), 'gims_pyramid_layout')
+    offs = np.zeros(max(n.value, 1), dtype=np.int64)
+    hs = np.zeros(max(n.value, 1), dtype=np.int32)
+    ws = np.zeros(max(n.value, 1), dtype=np.int32)
+    _lib.check(L.gims_pyramid_layout(h, w, cn, C.byref(n), offs.ctypes.data, hs.ctypes.data, ws.ctypes.data),
+               'gims_pyramid_layout')
+    nl = n.value
+    offs, hs, ws = offs[:nl], hs[:nl], ws[:nl]
+    total = int(offs[-1]) + int(hs[-1]) * int(ws[-1]) * cn if nl else 0
+    shapes = [(int(a), int(b)) for a, b in zip(hs, ws)]
+    # one upload: the level table (int64 offsets, int32 heights, int32 widths), then the image at a 256-byte boundary
+    img_at = (16 * nl + 255) // 256 * 256
+    st = torch.cuda.current_stream(dev)
+    with torch.cuda.device(dev):
+        buf = torch.empty(max(total, 1), dtype=torch.uint8, device=dev)
+        flat = _pinned_staging(img_at + img.size)
+        fl = flat.numpy()
+        fl[:8 * nl].view(np.int64)[:] = offs
+        fl[8 * nl:12 * nl].view(np.int32)[:] = hs
+        fl[12 * nl:16 * nl].view(np.int32)[:] = ws
+        np.copyto(fl[img_at:img_at + img.size].reshape(img.shape), img)
+        up = flat[:img_at + img.size].to(dev, non_blocking=True)
+        _STAGING.event = torch.cuda.Event()
+        _STAGING.event.record(st)                 # the staging buffer is reused by this thread's next call
+        d_off, d_h, d_w = up[:8 * nl].view(torch.int64), up[8 * nl:12 * nl].view(torch.int32), up[12 * nl:16 * nl].view(torch.int32)
+        if nl:
+            need = int(L.gims_pyramid_workspace_bytes(h, w, cn))
+            key = (str(dev), st.cuda_stream, __import__('threading').get_ident())
+            with _PYR_WS_LOCK:
+                wsp = _PYR_WS.get(key)
+            if wsp is None or wsp.numel() < need:
+                wsp = torch.empty(need, dtype=torch.uint8, device=dev)
+                with _PYR_WS_LOCK:
+                    _PYR_WS[key] = wsp
+            _lib.check(L.gims_gaussian_pyramid(_lib.ptr(up[img_at:]), h, w, cn, _lib.ptr(buf), _lib.ptr(wsp), wsp.numel(),
+                                               C.c_void_p(st.cuda_stream)), 'gims_gaussian_pyramid')
+    return DevicePyramid(buf, d_off, d_h, d_w, shapes, offs, cn)
+
+
 def extract_patches_device(kps, levels, device):
     """`extract_patches` on the GPU: (N, 32, 32[, C]) float32 ON `device`, bit-identical to the host path (the kernel follows
-    OpenCV's 8-bit fixed-point cubic warp, csrc/patches.cu).  The pyramid levels are uploaded once per image."""
+    OpenCV's 8-bit fixed-point cubic warp, csrc/patches.cu).  `levels`: the host pyramid (a list of uint8 arrays; the
+    levels that carry keypoints are uploaded) or a `DevicePyramid` of the same device (nothing is uploaded)."""
     import ctypes as C
     from . import _lib
     dev = torch.device(device)
     if dev.type != 'cuda':
         raise _lib.GimsError('extract_patches_device needs a CUDA device')
     n = len(kps)
-    cn = levels[0].shape[2] if levels[0].ndim == 3 else 1
-    shape = (n, PATCH_SIZE, PATCH_SIZE, cn) if levels[0].ndim == 3 else (n, PATCH_SIZE, PATCH_SIZE)
+    on_device = isinstance(levels, DevicePyramid)
+    if on_device:
+        pdev = levels.buffer.device
+        if dev.index is not None and dev.index != pdev.index:
+            raise _lib.GimsError('extract_patches_device: the pyramid is on %s, not %s' % (pdev, dev))
+        dev, cn = pdev, levels.channels
+        grey = cn == 1
+    else:
+        cn = levels[0].shape[2] if levels[0].ndim == 3 else 1
+        grey = levels[0].ndim != 3
+    shape = (n, PATCH_SIZE, PATCH_SIZE) if grey else (n, PATCH_SIZE, PATCH_SIZE, cn)
     out = torch.empty(shape, dtype=torch.float32, device=dev)
     if n == 0:
         return out
     level, inv = patch_maps(kps)
+    st = torch.cuda.current_stream(dev)
+    if on_device:
+        if int(level.max()) >= len(levels):
+            raise _lib.GimsError('extract_patches_device: a keypoint names level %d of a %d-level pyramid'
+                                 % (int(level.max()), len(levels)))
+        with torch.cuda.device(dev):
+            d_level = torch.from_numpy(level).to(dev)
+            d_inv = torch.from_numpy(inv).to(dev)
+            _lib.check(_lib.lib().gims_extract_patches(_lib.ptr(levels.buffer), _lib.ptr(levels.offset),
+                                                       _lib.ptr(levels.height), _lib.ptr(levels.width), len(levels), cn,
+                                                       _lib.ptr(d_level), _lib.ptr(d_inv), n, _lib.ptr(out),
+                                                       C.c_void_p(st.cuda_stream)), 'gims_extract_patches')
+        return out
     # only the levels that carry keypoints travel (the coarse octaves are small, the unused fine ones are not)
     used = np.zeros(len(levels), dtype=bool)
     used[level] = True
@@ -203,7 +316,6 @@ def extract_patches_device(kps, levels, device):
         if l.dtype != np.uint8:
             raise _lib.GimsError('extract_patches_device: pyramid levels must be uint8 (got %s)' % l.dtype)
         np.copyto(fl[o:o + l.size].reshape(l.shape), l)
-    st = torch.cuda.current_stream(dev)
     with torch.cuda.device(dev):
         d_lv = flat[:total].to(dev, non_blocking=True)
         _STAGING.event = torch.cuda.Event()
@@ -251,21 +363,31 @@ def describe(patches, carhynet, device, batch_size=512):
     return d.to(device)
 
 
-def host_stages(image_sets, max_kp=-1):
+def device_pyramids(images, device):
+    """Enqueue `gaussian_pyramid_device` for every image of `images` that it takes (uint8, 1 or 3 channels) when `device`
+    is a CUDA device and GIMS_HOST_PATCHES is not 1; None for the others, whose pyramid stays on the host."""
+    on_gpu = torch.device(device).type == 'cuda' and os.environ.get('GIMS_HOST_PATCHES') != '1'
+    return [gaussian_pyramid_device(img, device) if on_gpu and pyramid_on_device(img) else None for img in images]
+
+
+def host_stages(image_sets, max_kp=-1, pyramids=None):
     """The OpenCV stages (SIFT detection + Gaussian pyramid) of several images side by side — OpenCV releases the GIL, and
     the reference runs image 0 and image 1 one after the other (matching.py:18-24).  `image_sets`: a list of iterables of
-    images (each what `data['image']` is); returns, per set, a list of (keypoints, pyramid levels)."""
+    images (each what `data['image']` is); returns, per set, a list of (keypoints, pyramid levels).  `pyramids`, if given,
+    holds per set and image a pyramid already built (a `DevicePyramid`) or None: only the None ones are built here."""
     flat = [np.asarray(img) for imgs in image_sets for img in imgs]
     counts = [len(imgs) for imgs in image_sets]
+    pyrs = [p for ps in pyramids for p in ps] if pyramids is not None else [None] * len(flat)
 
-    def stage(img):
-        return detect(img, max_kp), gaussian_pyramid(img)
+    def stage(args):
+        img, pyr = args
+        return detect(img, max_kp), (gaussian_pyramid(img) if pyr is None else pyr)
     if len(flat) > 1:
         from concurrent.futures import ThreadPoolExecutor
         with ThreadPoolExecutor(max_workers=min(len(flat), 8)) as pool:
-            done = list(pool.map(stage, flat))
+            done = list(pool.map(stage, zip(flat, pyrs)))
     else:
-        done = [stage(img) for img in flat]
+        done = [stage(a) for a in zip(flat, pyrs)]
     out, i = [], 0
     for c in counts:
         out.append(done[i:i + c])
@@ -277,15 +399,19 @@ def sift_forward(data, device, staged=None):
     """Same dict in / dict out as utils/common.py:837-893: `data['image']` iterates over images, `data['carhynet']` is the
     caller's descriptor object; returns lists (one entry per image) of device tensors
     `keypoints` (N, 2) fp32 pixel xy, `scores` (N,) fp32 SIFT responses, `descriptors` (256, N) fp32.
-    `staged`: the (keypoints, pyramid) pairs of the images if `host_stages` has already produced them."""
+    `staged`: the (keypoints, pyramid) pairs of the images if `host_stages` has already produced them.  On a CUDA device
+    the pyramid of a uint8 grey or colour image is built there (enqueued before detection starts, so the two overlap)."""
     max_kp = data.get('max_keypoints', -1)
     kpts, scores, descs = [], [], []
     images = [np.asarray(img) for img in data['image']]
     if staged is None:
-        staged = host_stages([images], max_kp)[0]
+        staged = host_stages([images], max_kp, [device_pyramids(images, device)])[0]
     for img, (kps, levels) in zip(images, staged):
-        on_gpu = torch.device(device).type == 'cuda' and levels[0].dtype == np.uint8 and os.environ.get('GIMS_HOST_PATCHES') != '1'
-        patches = extract_patches_device(kps, levels, device) if on_gpu else extract_patches(kps, levels)
+        if isinstance(levels, DevicePyramid):
+            patches = extract_patches_device(kps, levels, device)
+        else:
+            on_gpu = torch.device(device).type == 'cuda' and levels[0].dtype == np.uint8 and os.environ.get('GIMS_HOST_PATCHES') != '1'
+            patches = extract_patches_device(kps, levels, device) if on_gpu else extract_patches(kps, levels)
         d = describe(patches, data['carhynet'], device)                        # (N, 128), on the device
         pts = np.array([k.pt for k in kps], dtype=np.float32).reshape(-1, 2)
         resp = np.array([k.response for k in kps], dtype=np.float32)

@@ -1,7 +1,8 @@
 """Host-side mirror of the reference's `Matching` front-end (models/matching.py:8-30)."""
+import numpy as np
 import torch
 
-from .frontend import host_stages, sift_forward
+from .frontend import device_pyramids, host_stages, sift_forward
 from .gmatcher import GMatcher
 
 
@@ -10,7 +11,8 @@ class Matching(torch.nn.Module):
 
     With `keypoints{0,1}` in `data` the matcher runs on them directly (matching.py:17,21); without, the images go
     through `sift_forward` first (matching.py:18-24 -> utils/common.py:837-893; here gims_b200/frontend.py: OpenCV SIFT
-    and patches on the host, the caller's CAR-HyNet on the device, descriptors never leave it).
+    on the host while the Gaussian pyramid is built on the device, patches and the caller's CAR-HyNet on the device,
+    descriptors never leave it).
     """
 
     def __init__(self, config={}):
@@ -21,10 +23,13 @@ class Matching(torch.nn.Module):
     def forward(self, data):
         pred = {}
         need = [s for s in ('0', '1') if 'keypoints' + s not in data]
-        # the OpenCV stages of both images run side by side (the reference does image 0, then image 1)
-        staged = dict(zip(need, host_stages([data['image' + s] for s in need], self.max_keypoints))) if need else {}
+        dev = data.get('device', self.gmodel.bin_score.device)
+        # the pyramids go onto the caller's stream first (uint8 grey / colour images, CUDA device); the OpenCV stages of
+        # both images then run side by side (the reference does image 0, then image 1)
+        images = [[np.asarray(img) for img in data['image' + s]] for s in need]
+        pyramids = [device_pyramids(imgs, dev) for imgs in images]
+        staged = dict(zip(need, host_stages(images, self.max_keypoints, pyramids))) if need else {}
         for s in need:
-            dev = data.get('device', self.gmodel.bin_score.device)
             out = sift_forward({'image': data['image' + s], 'max_keypoints': self.max_keypoints,
                                 'carhynet': data['carhynet']}, device=dev, staged=staged[s])
             pred = {**pred, **{k + s: v for k, v in out.items()}}

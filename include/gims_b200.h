@@ -234,7 +234,8 @@ GIMS_API int gims_sinkhorn_match(const float* couplings, int ld, int n0_max, int
 /* ---- front end: oriented keypoint patches on the device (SURVEY.md §8f row 2) ------------------
  * replaces the per-keypoint loop of ComputePatches (utils/library.py:84-110: cv2.warpAffine INTER_CUBIC / BORDER_CONSTANT
  * into 64 x 64) and the INTER_AREA resize to 32 x 32 + /255 of utils/common.py:882-884; bit-identical to OpenCV's 8-bit
- * fixed-point warp.  The Gaussian pyramid (utils/library.py:234-293) is built by the caller (OpenCV) and uploaded:
+ * fixed-point warp.  The Gaussian pyramid (utils/library.py:234-293) is gims_gaussian_pyramid's output (below) or built by
+ * the caller (OpenCV) and uploaded:
  *   levels           uint8, every level H x W x channels (channels 1 or 3), concatenated; level l starts at byte
  *                    level_offset_dev[l] and is level_height_dev[l] x level_width_dev[l]
  *   kp_level_dev     [n_kp] pyramid level of each keypoint ((octave - firstOctave) * (nOctaveLayers + 3) + layer)
@@ -247,6 +248,25 @@ GIMS_API int gims_extract_patches(const unsigned char* levels, const long long* 
 
 /* test hook: the 32 x 32 x 16 int16 bicubic weight table of gims_extract_patches, as built on the host */
 GIMS_API int gims_debug_bicubic_table(short* out_host);
+
+/* ---- front end: the Gaussian pyramid the patches are cut from, on the device ---------------------------------------
+ * replaces frontend.gaussian_pyramid (utils/library.py:234-293: cv2.resize x2 INTER_LINEAR_EXACT, per octave five
+ * cv2.GaussianBlur with the incremental SIFT sigmas, each next octave seeded by INTER_NEAREST x0.5 of level 3); byte for
+ * byte what OpenCV's 8-bit fixed-point arithmetic gives.  `image` is h x w x channels uint8 (channels 1 or 3, interleaved).
+ * gims_pyramid_layout (host only) gives the level count, nOctaves * 6 with
+ * nOctaves = round_half_even(log(float32(min(2h, 2w))) / log(2) - 2) + 1, and, for each level, its byte offset inside the
+ * level buffer and its size: the level table gims_extract_patches takes.  The three arrays may be null (call once to get
+ * the count); each one that is not null must hold n_levels entries.  The buffer holds
+ * offset_host[n - 1] + height_host[n - 1] * width_host[n - 1] * channels bytes.
+ * gims_gaussian_pyramid writes every level into `levels_out` in that layout; the workspace holds the uint16 row pass. */
+GIMS_API int gims_pyramid_layout(int h, int w, int channels, int* n_levels, int64_t* offset_host, int* height_host,
+                        int* width_host);
+GIMS_API size_t gims_pyramid_workspace_bytes(int h, int w, int channels);
+GIMS_API int gims_gaussian_pyramid(const unsigned char* image, int h, int w, int channels, unsigned char* levels_out,
+                          void* workspace, size_t workspace_bytes, void* stream);
+
+/* test hook: the 8-bit fixed-point taps (sum 256) cv2.GaussianBlur uses for `sigma`; taps_host holds at least 127 ints */
+GIMS_API int gims_debug_gaussian_kernel(double sigma, int* taps_host, int* n_host);
 
 /* ---- caller-side result consumption on the device (SURVEY.md §8f row 3) --------------------
  * gims_gt_matches replaces utils/preprocess_utils.py:98-132 torch_find_matches (called at eval_homography.py:205):
