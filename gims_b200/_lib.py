@@ -19,6 +19,7 @@ STATUS_SINKHORN_EXACT = 0x200
 GEMM_SIMT, GEMM_TC, GEMM_TC_F16, GEMM_BF16 = 0, 1, 2, 3
 GEMM_MODES = {'simt': GEMM_SIMT, 'tf32': GEMM_TC, 'tc': GEMM_TC, 'f16': GEMM_TC_F16, 'bf16': GEMM_BF16}
 STATUS_FP16_RANGE = 4
+STATUS_KEYPOINT_OVERFLOW = 8
 PROF = {'gemm': 1, 'attention': 2, 'sinkhorn': 3, 'score': 4, 'cosine': 5, 'sage_gather': 6}
 
 
@@ -136,6 +137,10 @@ SIGNATURES = {
     'gims_gaussian_pyramid': (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_size_t,
                                         C.c_void_p]),
     'gims_debug_gaussian_kernel': (C.c_int, [C.c_double, C.c_void_p, C.POINTER(C.c_int)]),
+    'gims_sift_workspace_bytes': (C.c_size_t, [C.c_int, C.c_int, C.c_int, C.c_int]),
+    'gims_sift_detect': (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_size_t,
+                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                   C.c_void_p]),
     'gims_gt_workspace_bytes': (C.c_size_t, [C.c_int, C.c_int]),
     'gims_gt_matches': (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_float, C.c_int, C.c_void_p,
                                   C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -8,7 +8,8 @@ Mirrors `sift_forward` (utils/common.py:837-893): OpenCV SIFT detection, OpenCV-
 128-d descriptor duplicated to 256-d (utils/common.py:891).
 
 What is different from the reference, and why:
-  * detection stays on the host (OpenCV); the Gaussian pyramid of a uint8 grey or colour image is built on the device,
+  * detection stays on the host (OpenCV) by default; `Matching({'detector': 'device'})` detects on the GPU instead
+    (`detect_device`, csrc/sift.cu: within a tolerance of cv2, not bit for bit, see DESIGN.md §9); the Gaussian pyramid of a uint8 grey or colour image is built on the device,
     byte for byte what OpenCV builds (`gaussian_pyramid_device`, csrc/pyramid.cu), while the host detects; the per-keypoint patch loop (§8f row 2: cv2.warpAffine
     + resize per keypoint, 200-500 ms per image) runs as ONE kernel on the device that reproduces OpenCV's fixed-point
     cubic warp bit for bit (`extract_patches_device`, csrc/patches.cu; GIMS_HOST_PATCHES=1 keeps the host loop);
@@ -119,21 +120,35 @@ def extract_patches(kps, levels, support=PATCH_SUPPORT, out_size=PATCH_SIZE):
     return np.array(out) / 255.0
 
 
+def keypoint_arrays(kps):
+    """(pt float64 [N, 2], size, angle float64 [N], octave int64 [N]) of a list of cv2.KeyPoint."""
+    n = len(kps)
+    return (np.array([k.pt for k in kps], dtype=np.float64).reshape(n, 2),
+            np.array([k.size for k in kps], dtype=np.float64).reshape(n),
+            np.array([k.angle for k in kps], dtype=np.float64).reshape(n),
+            np.array([k.octave for k in kps], dtype=np.int64).reshape(n))
+
+
 def patch_maps(kps):
+    """`patch_maps_from_arrays` of a list of cv2.KeyPoint."""
+    return patch_maps_from_arrays(*keypoint_arrays(kps))
+
+
+def patch_maps_from_arrays(pt, size, angle, octave):
     """Per keypoint: the pyramid level index and the 2 x 3 matrix `extract_patches` hands to cv2.warpAffine
     (utils/library.py:84-110), vectorised over the keypoints with the reference's dtypes (float32 rotation / step, float64
-    shift), then inverted the way cv::warpAffine inverts its argument (imgwarp.cpp).  Returns (level int32 [N],
-    inverse map float64 [N, 6])."""
-    n = len(kps)
+    shift), then inverted the way cv::warpAffine inverts its argument (imgwarp.cpp).  `pt` (N, 2), `size`, `angle`,
+    `octave` (N,) as cv2.KeyPoint holds them.  Returns (level int32 [N], inverse map float64 [N, 6])."""
+    n = len(size)
     r = (PATCH_SUPPORT - 1) / 2
-    octv = np.array([k.octave for k in kps], dtype=np.int64).reshape(n)
+    octv = np.asarray(octave, dtype=np.int64).reshape(n)
     octave = octv & 0xFF
     layer = (octv >> 8) & 0xFF
     octave = np.where(octave >= 128, octave - 256, octave)
     scale = np.where(octave >= 0, 1.0 / (1 << np.maximum(octave, 0)), (1 << np.maximum(-octave, 0)).astype(np.float64))
-    size = np.array([k.size for k in kps], dtype=np.float64).reshape(n)
-    pt = np.array([k.pt for k in kps], dtype=np.float64).reshape(n, 2)
-    ang = np.array([k.angle for k in kps], dtype=np.float64).reshape(n)
+    size = np.asarray(size, dtype=np.float64).reshape(n)
+    pt = np.asarray(pt, dtype=np.float64).reshape(n, 2)
+    ang = np.asarray(angle, dtype=np.float64).reshape(n)
     step = size * scale * 0.5
     centre = pt * scale[:, None]
     angle = 360.0 - ang
@@ -178,11 +193,12 @@ def _pinned_staging(nbytes):
 class DevicePyramid:
     """The Gaussian pyramid of one image on the device (`gaussian_pyramid_device`): every level in one uint8 buffer and
     the level table `gims_extract_patches` reads.  `buffer` uint8, `offset` int64, `height` / `width` int32 are device
-    tensors; `shapes` is the host copy of the level sizes."""
+    tensors; `shapes` is the host copy of the level sizes; `image` is the uploaded image (uint8, on the device), which
+    `detect_device` reuses."""
 
-    def __init__(self, buffer, offset, height, width, shapes, offsets, channels):
+    def __init__(self, buffer, offset, height, width, shapes, offsets, channels, image=None):
         self.buffer, self.offset, self.height, self.width = buffer, offset, height, width
-        self.shapes, self.offsets, self.channels = shapes, offsets, channels
+        self.shapes, self.offsets, self.channels, self.image = shapes, offsets, channels, image
 
     def __len__(self):
         return len(self.shapes)
@@ -261,13 +277,14 @@ def gaussian_pyramid_device(image, device):
                     _PYR_WS[key] = wsp
             _lib.check(L.gims_gaussian_pyramid(_lib.ptr(up[img_at:]), h, w, cn, _lib.ptr(buf), _lib.ptr(wsp), wsp.numel(),
                                                C.c_void_p(st.cuda_stream)), 'gims_gaussian_pyramid')
-    return DevicePyramid(buf, d_off, d_h, d_w, shapes, offs, cn)
+    return DevicePyramid(buf, d_off, d_h, d_w, shapes, offs, cn, up[img_at:])
 
 
 def extract_patches_device(kps, levels, device):
     """`extract_patches` on the GPU: (N, 32, 32[, C]) float32 ON `device`, bit-identical to the host path (the kernel follows
     OpenCV's 8-bit fixed-point cubic warp, csrc/patches.cu).  `levels`: the host pyramid (a list of uint8 arrays; the
-    levels that carry keypoints are uploaded) or a `DevicePyramid` of the same device (nothing is uploaded)."""
+    levels that carry keypoints are uploaded) or a `DevicePyramid` of the same device (nothing is uploaded).  `kps`: a list
+    of cv2.KeyPoint or the `DeviceKeypoints` of `detect_device`."""
     import ctypes as C
     from . import _lib
     dev = torch.device(device)
@@ -288,7 +305,7 @@ def extract_patches_device(kps, levels, device):
     out = torch.empty(shape, dtype=torch.float32, device=dev)
     if n == 0:
         return out
-    level, inv = patch_maps(kps)
+    level, inv = patch_maps_from_arrays(*kps.host()) if isinstance(kps, DeviceKeypoints) else patch_maps(kps)
     st = torch.cuda.current_stream(dev)
     if on_device:
         if int(level.max()) >= len(levels):
@@ -395,6 +412,118 @@ def host_stages(image_sets, max_kp=-1, pyramids=None):
     return out
 
 
+SIFT_KP_CAP = 16384             # first keypoint capacity of detect_device; 4x more on each overflow
+_SIFT_WS = {}                   # (device, stream, thread) -> grow-only uint8 workspace of gims_sift_detect
+_SIFT_WS_LOCK = __import__('threading').Lock()
+
+
+class DeviceKeypoints:
+    """The keypoints `detect_device` found in one image, on the device: `pt` (N, 2), `size`, `angle`, `response` float32
+    and `octave` int32 (packed as cv2.KeyPoint.octave), in cv2's order (see gims_sift_detect).  `host()` gives the same
+    records as numpy arrays (pt, size, angle, octave), read back once with the count."""
+
+    def __init__(self, n, pt, size, angle, response, octave, host):
+        self.n, self.pt, self.size, self.angle, self.response, self.octave = n, pt, size, angle, response, octave
+        self._host = host
+
+    def __len__(self):
+        return self.n
+
+    def host(self):
+        return self._host
+
+    def keypoints(self):
+        """The records as a list of cv2.KeyPoint."""
+        cv2 = _cv2()
+        pt, size, angle, octave = self._host
+        resp = self.response.cpu().numpy()
+        return [cv2.KeyPoint(float(pt[i, 0]), float(pt[i, 1]), float(size[i]), float(angle[i]), float(resp[i]),
+                             int(octave[i])) for i in range(self.n)]
+
+
+class _PendingDetect:
+    """A detection enqueued by `detect_enqueue`: the device outputs and their pinned host copy, not yet waited for."""
+
+    def __init__(self, image, h, w, cn, dev, max_keypoints, kp_cap):
+        import ctypes as C
+        from . import _lib
+        self.args = (image, h, w, cn, dev, max_keypoints)
+        self.cap = kp_cap
+        L = _lib.lib()
+        st = torch.cuda.current_stream(dev)
+        with torch.cuda.device(dev):
+            # one buffer: count, status, 2 spare ints, then pt [cap][2], size, angle, response, octave
+            out = torch.zeros(4 + 6 * kp_cap, dtype=torch.int32, device=dev)
+            f = out.view(torch.float32)
+            self.pt = f[4:4 + 2 * kp_cap].view(kp_cap, 2)
+            self.size, self.angle, self.response = (f[4 + k * kp_cap:4 + (k + 1) * kp_cap] for k in (2, 3, 4))
+            self.octave = out[4 + 5 * kp_cap:]
+            need = int(L.gims_sift_workspace_bytes(h, w, cn, kp_cap))
+            key = (str(dev), st.cuda_stream, __import__('threading').get_ident())
+            with _SIFT_WS_LOCK:
+                wsp = _SIFT_WS.get(key)
+            if wsp is None or wsp.numel() < need:
+                wsp = torch.empty(need, dtype=torch.uint8, device=dev)
+                with _SIFT_WS_LOCK:
+                    _SIFT_WS[key] = wsp
+            _lib.check(L.gims_sift_detect(_lib.ptr(image), h, w, cn, max_keypoints, kp_cap, _lib.ptr(wsp), wsp.numel(),
+                                          _lib.ptr(self.pt), _lib.ptr(self.size), _lib.ptr(self.angle),
+                                          _lib.ptr(self.response), _lib.ptr(self.octave), _lib.ptr(out[0:1]),
+                                          _lib.ptr(out[1:2]), C.c_void_p(st.cuda_stream)), 'gims_sift_detect')
+            self.host = torch.empty(out.numel(), dtype=torch.int32, pin_memory=True)
+            self.host.copy_(out, non_blocking=True)
+            self.done = torch.cuda.Event()
+            self.done.record(st)
+        self.out = out
+
+    def result(self):
+        """Wait for the read-back; on GIMS_STATUS_KEYPOINT_OVERFLOW run again with 4x the capacity."""
+        from . import _lib
+        self.done.synchronize()
+        hv = self.host.numpy()
+        status = int(hv[1])
+        if status & _lib.STATUS_KEYPOINT_OVERFLOW:
+            return _PendingDetect(*self.args, kp_cap=4 * self.cap).result()
+        if status & _lib.STATUS_ERROR_MASK:
+            raise _lib.GimsError('gims_sift_detect: status 0x%x' % status)
+        n, cap = int(hv[0]), self.cap
+        hf = hv.view(np.float32)
+        host = (hf[4:4 + 2 * n].reshape(n, 2).astype(np.float64), hf[4 + 2 * cap:4 + 2 * cap + n].astype(np.float64),
+                hf[4 + 3 * cap:4 + 3 * cap + n].astype(np.float64), hv[4 + 5 * cap:4 + 5 * cap + n].astype(np.int64))
+        return DeviceKeypoints(n, self.pt[:n], self.size[:n], self.angle[:n], self.response[:n], self.octave[:n], host)
+
+
+def detect_enqueue(image, device, max_keypoints=-1, pyramid=None, kp_cap=SIFT_KP_CAP):
+    """Enqueue `detect_device` on the current stream of `device` without waiting; `.result()` of the returned object
+    waits and gives the `DeviceKeypoints`.  `pyramid`: the `DevicePyramid` of the same image, whose uploaded copy is
+    reused (otherwise the image is uploaded here)."""
+    from . import _lib
+    dev = torch.device(device)
+    if dev.type != 'cuda':
+        raise _lib.GimsError('detect_device needs a CUDA device')
+    img = np.asarray(image)
+    if not pyramid_on_device(img):
+        raise _lib.GimsError('detect_device: need a uint8 (H, W), (H, W, 1) or (H, W, 3) image (got %s %s)'
+                             % (img.dtype, img.shape))
+    h, w = img.shape[:2]
+    cn = 3 if img.ndim == 3 and img.shape[2] == 3 else 1
+    if pyramid is not None and pyramid.image is not None:
+        d_img = pyramid.image
+        dev = d_img.device
+    else:
+        with torch.cuda.device(dev):
+            d_img = torch.from_numpy(np.ascontiguousarray(img).reshape(-1)).pin_memory().to(dev, non_blocking=True)
+    return _PendingDetect(d_img, h, w, cn, dev, int(max_keypoints), int(kp_cap))
+
+
+def detect_device(image, device, max_keypoints=-1, pyramid=None):
+    """`detect` on the GPU (csrc/sift.cu): SIFT keypoints of a uint8 grey or colour image as `DeviceKeypoints`, the
+    strongest `max_keypoints` first if that limit is positive.  Not bit-identical to cv2 (cv2 is not bit-identical to
+    itself): the records equal oracle/cv_sift_oracle.py bit for bit and agree with cv2 within 0.01 px, 1e-3 relative size
+    and 0.5 degrees for more than 99 % of keypoints.  Waits for the count and the records (one read-back)."""
+    return detect_enqueue(image, device, max_keypoints, pyramid).result()
+
+
 def sift_forward(data, device, staged=None):
     """Same dict in / dict out as utils/common.py:837-893: `data['image']` iterates over images, `data['carhynet']` is the
     caller's descriptor object; returns lists (one entry per image) of device tensors
@@ -413,9 +542,13 @@ def sift_forward(data, device, staged=None):
             on_gpu = torch.device(device).type == 'cuda' and levels[0].dtype == np.uint8 and os.environ.get('GIMS_HOST_PATCHES') != '1'
             patches = extract_patches_device(kps, levels, device) if on_gpu else extract_patches(kps, levels)
         d = describe(patches, data['carhynet'], device)                        # (N, 128), on the device
-        pts = np.array([k.pt for k in kps], dtype=np.float32).reshape(-1, 2)
-        resp = np.array([k.response for k in kps], dtype=np.float32)
-        kpts.append(torch.from_numpy(pts).to(device))
-        scores.append(torch.from_numpy(resp).to(device))
+        if isinstance(kps, DeviceKeypoints):
+            kpts.append(kps.pt)
+            scores.append(kps.response)
+        else:
+            pts = np.array([k.pt for k in kps], dtype=np.float32).reshape(-1, 2)
+            resp = np.array([k.response for k in kps], dtype=np.float32)
+            kpts.append(torch.from_numpy(pts).to(device))
+            scores.append(torch.from_numpy(resp).to(device))
         descs.append(torch.cat([d, d], dim=1).t().contiguous())                # utils/common.py:891
     return {'keypoints': kpts, 'scores': scores, 'descriptors': descs}

@@ -62,6 +62,7 @@ extern "C" {
 #define GIMS_STATUS_EDGE_OVERFLOW     1u   /* edge_cap exceeded: the graph is reported EMPTY (N' = 0), retry larger */
 #define GIMS_STATUS_SINKHORN_TIMEOUT  2u   /* a bounded poll inside k_sinkhorn expired: outputs are poisoned (NaN / -2) */
 #define GIMS_STATUS_FP16_RANGE        4u   /* GIMS_GEMM_TC_F16: a tensor-core operand reached 32768 — rerun with GIMS_GEMM_TC */
+#define GIMS_STATUS_KEYPOINT_OVERFLOW 8u   /* gims_sift_detect: kp_cap exceeded, no keypoints reported — retry larger */
 #define GIMS_STATUS_ERROR_MASK        0xffu
 /* Information bits: which Sinkhorn iteration the launch ran */
 #define GIMS_STATUS_SINKHORN_FAST   0x100u /* exp-free scaled-kernel iteration */
@@ -267,6 +268,24 @@ GIMS_API int gims_gaussian_pyramid(const unsigned char* image, int h, int w, int
 
 /* test hook: the 8-bit fixed-point taps (sum 256) cv2.GaussianBlur uses for `sigma`; taps_host holds at least 127 ints */
 GIMS_API int gims_debug_gaussian_kernel(double sigma, int* taps_host, int* n_host);
+
+/* ---- front end: SIFT keypoint detection on the device --------------------------------------------------------------
+ * OpenCV 4.x SIFT::detect with frontend.SIFT_CONFIG (3 layers, contrastThreshold 0.001, edgeThreshold 80, sigma 1.6,
+ * the image doubled first) on the float32 scale space of the grey image, in the float32 order of operations that
+ * oracle/cv_sift_oracle.py fixes: the records equal that restatement bit for bit and agree with cv2 within a tolerance
+ * (cv2 does not reproduce itself bit for bit).  The octave count is gims_pyramid_layout's, so the keypoints index the
+ * patch pyramid.  `image` is h x w x channels uint8 (channels 1 or 3, BGR), on the device.
+ * Outputs (kp_cap entries each, on the device): pt [kp_cap][2] float xy in input pixels, size, angle (degrees), response
+ * float, octave int32 packed as cv2.KeyPoint.octave; *n_kp_dev the number written.  The order is cv2's (sorted by x, y,
+ * -size, angle, -response, -octave, duplicates of (pt, size, angle) removed); with max_keypoints > 0 and more keypoints
+ * than that, the max_keypoints strongest by response, strongest first, ties in that sorted order.
+ * kp_cap bounds the keypoints before duplicates are removed; the scale-space extrema are bounded by 2 * kp_cap.  When
+ * either bound is exceeded GIMS_STATUS_KEYPOINT_OVERFLOW is OR-ed into *status_dev and *n_kp_dev is 0: retry with a
+ * larger kp_cap.  Enqueue-only on `stream`; the workspace holds gims_sift_workspace_bytes(h, w, channels, kp_cap). */
+GIMS_API size_t gims_sift_workspace_bytes(int h, int w, int channels, int kp_cap);
+GIMS_API int gims_sift_detect(const unsigned char* image, int h, int w, int channels, int max_keypoints, int kp_cap,
+                     void* workspace, size_t workspace_bytes, float* pt, float* size, float* angle, float* response,
+                     int* octave, int* n_kp_dev, unsigned* status_dev, void* stream);
 
 /* ---- caller-side result consumption on the device (SURVEY.md §8f row 3) --------------------
  * gims_gt_matches replaces utils/preprocess_utils.py:98-132 torch_find_matches (called at eval_homography.py:205):
