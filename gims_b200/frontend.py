@@ -20,11 +20,16 @@ What is different from the reference, and why:
 The caller's `carhynet` object is used as it is: anything with a `.model` (the torch module) is run directly; an object
 that only offers the reference's `compute_sift(patches, kps, color)` is called through that method.
 """
+import ctypes as C
 import math
 import os
+import threading
+from concurrent.futures import ThreadPoolExecutor
 
 import numpy as np
 import torch
+
+from . import _lib
 
 # the constants sift_forward hard-codes (utils/common.py:838-848)
 SIFT_CONFIG = dict(nfeatures=None, nOctaveLayers=3, contrastThreshold=0.001, edgeThreshold=80, sigma=1.6)
@@ -175,19 +180,47 @@ def patch_maps_from_arrays(pt, size, angle, octave):
     return level, np.ascontiguousarray(inv, dtype=np.float64)
 
 
-_STAGING = __import__('threading').local()
+def _check_levels(level, n_levels):
+    """Raise GimsError unless every level index of `patch_maps_from_arrays` names one of `n_levels` pyramid levels: a
+    packed octave below FIRST_OCTAVE gives a negative index, one past the coarsest octave an index past the end, and the
+    patch kernel would read outside its level table."""
+    bad = level[(level < 0) | (level >= n_levels)]
+    if len(bad):
+        raise _lib.GimsError('extract_patches_device: a keypoint names level %d of a %d-level pyramid' % (bad[0], n_levels))
 
 
-def _pinned_staging(nbytes):
-    """Grow-only pinned host buffer of the calling thread (pinning 40 MB per call cost more than the copy itself)."""
+_STAGING = threading.local()
+
+
+def _pinned_upload(parts, nbytes, dev):
+    """A new uint8 tensor of `nbytes` on `dev`, copied on its current stream from the calling thread's grow-only pinned
+    buffer (pinning 40 MB per call cost more than the copy itself), into which `parts`, (byte offset, array) pairs, are
+    written first.  The buffer's previous upload is waited for before it is overwritten."""
     ev = getattr(_STAGING, 'event', None)
     if ev is not None:
-        ev.synchronize()                          # the previous upload from this buffer has left the host
+        ev.synchronize()
     buf = getattr(_STAGING, 'buf', None)
     if buf is None or buf.numel() < nbytes:
         buf = torch.empty(max(nbytes, 1 << 20), dtype=torch.uint8).pin_memory()
         _STAGING.buf = buf
-    return buf
+    host = buf.numpy()
+    for at, a in parts:
+        np.copyto(host[at:at + a.nbytes].view(a.dtype).reshape(a.shape), a)
+    up = buf[:nbytes].to(dev, non_blocking=True)
+    _STAGING.event = torch.cuda.Event()
+    _STAGING.event.record(torch.cuda.current_stream(dev))
+    return up
+
+
+def _upload_level_table(offs, hs, ws, parts, nbytes, dev):
+    """One `_pinned_upload` of a level table (int64 offsets, int32 heights, int32 widths) and, at the next 256-byte
+    boundary, the `nbytes` the `parts` describe (offsets relative to that boundary).  Returns the device tensors
+    (data, offset, height, width)."""
+    nl = len(offs)
+    at = (16 * nl + 255) // 256 * 256
+    up = _pinned_upload([(0, offs), (8 * nl, hs), (12 * nl, ws)] + [(at + o, a) for o, a in parts], at + nbytes, dev)
+    return (up[at:], up[:8 * nl].view(torch.int64), up[8 * nl:12 * nl].view(torch.int32),
+            up[12 * nl:16 * nl].view(torch.int32))
 
 
 class DevicePyramid:
@@ -211,14 +244,23 @@ class DevicePyramid:
         return v.view(h, w, self.channels) if self.channels == 3 else v.view(h, w)
 
 
-_PYR_WS = {}                    # (device, stream, thread) -> grow-only uint8 workspace of gims_gaussian_pyramid
-_PYR_WS_LOCK = __import__('threading').Lock()
-
-
 def pyramid_on_device(image):
-    """True if `gaussian_pyramid_device` can build this image's pyramid: uint8, grey or 3-channel colour."""
+    """True if the device kernels take this image (`gaussian_pyramid_device`, `detect_device`): uint8, grey or 3-channel
+    colour."""
     a = np.asarray(image)
     return a.dtype == np.uint8 and (a.ndim == 2 or (a.ndim == 3 and a.shape[2] in (1, 3))) and a.size > 0
+
+
+def _device_image(image, device, what):
+    """(array, h, w, channels) of an image the device kernels take; GimsError naming `what` if `device` is not a CUDA
+    device or the image is not uint8 with 1 or 3 channels."""
+    if torch.device(device).type != 'cuda':
+        raise _lib.GimsError('%s needs a CUDA device' % what)
+    img = np.asarray(image)
+    if not pyramid_on_device(img):
+        raise _lib.GimsError('%s: need a uint8 (H, W), (H, W, 1) or (H, W, 3) image (got %s %s)'
+                             % (what, img.dtype, img.shape))
+    return img, img.shape[0], img.shape[1], 3 if img.ndim == 3 and img.shape[2] == 3 else 1
 
 
 def gaussian_pyramid_device(image, device):
@@ -226,19 +268,9 @@ def gaussian_pyramid_device(image, device):
     resize and blur).  Only the image travels: it is copied through the calling thread's pinned staging buffer and the
     pyramid is enqueued on the current stream of `device`; nothing waits for it.  Returns a `DevicePyramid`, which
     `extract_patches_device` takes in place of host levels.  The level buffer belongs to the returned object (the
-    pyramids of several images may be alive at once); the row-pass workspace is cached per (device, stream, thread),
-    grow-only, and its reuse is ordered by the stream."""
-    import ctypes as C
-    from . import _lib
+    pyramids of several images may be alive at once); the row-pass workspace is allocated per call on the stream."""
+    img, h, w, cn = _device_image(image, device, 'gaussian_pyramid_device')
     dev = torch.device(device)
-    if dev.type != 'cuda':
-        raise _lib.GimsError('gaussian_pyramid_device needs a CUDA device')
-    img = np.asarray(image)
-    if not pyramid_on_device(img):
-        raise _lib.GimsError('gaussian_pyramid_device: need a uint8 (H, W), (H, W, 1) or (H, W, 3) image (got %s %s)'
-                             % (img.dtype, img.shape))
-    h, w = img.shape[:2]
-    cn = 3 if img.ndim == 3 and img.shape[2] == 3 else 1
     L = _lib.lib()
     n = C.c_int(0)
     _lib.check(L.gims_pyramid_layout(h, w, cn, C.byref(n), None, None, None), 'gims_pyramid_layout')
@@ -251,48 +283,28 @@ def gaussian_pyramid_device(image, device):
     offs, hs, ws = offs[:nl], hs[:nl], ws[:nl]
     total = int(offs[-1]) + int(hs[-1]) * int(ws[-1]) * cn if nl else 0
     shapes = [(int(a), int(b)) for a, b in zip(hs, ws)]
-    # one upload: the level table (int64 offsets, int32 heights, int32 widths), then the image at a 256-byte boundary
-    img_at = (16 * nl + 255) // 256 * 256
-    st = torch.cuda.current_stream(dev)
     with torch.cuda.device(dev):
         buf = torch.empty(max(total, 1), dtype=torch.uint8, device=dev)
-        flat = _pinned_staging(img_at + img.size)
-        fl = flat.numpy()
-        fl[:8 * nl].view(np.int64)[:] = offs
-        fl[8 * nl:12 * nl].view(np.int32)[:] = hs
-        fl[12 * nl:16 * nl].view(np.int32)[:] = ws
-        np.copyto(fl[img_at:img_at + img.size].reshape(img.shape), img)
-        up = flat[:img_at + img.size].to(dev, non_blocking=True)
-        _STAGING.event = torch.cuda.Event()
-        _STAGING.event.record(st)                 # the staging buffer is reused by this thread's next call
-        d_off, d_h, d_w = up[:8 * nl].view(torch.int64), up[8 * nl:12 * nl].view(torch.int32), up[12 * nl:16 * nl].view(torch.int32)
+        d_img, d_off, d_h, d_w = _upload_level_table(offs, hs, ws, [(0, img)], img.size, dev)
         if nl:
-            need = int(L.gims_pyramid_workspace_bytes(h, w, cn))
-            key = (str(dev), st.cuda_stream, __import__('threading').get_ident())
-            with _PYR_WS_LOCK:
-                wsp = _PYR_WS.get(key)
-            if wsp is None or wsp.numel() < need:
-                wsp = torch.empty(need, dtype=torch.uint8, device=dev)
-                with _PYR_WS_LOCK:
-                    _PYR_WS[key] = wsp
-            _lib.check(L.gims_gaussian_pyramid(_lib.ptr(up[img_at:]), h, w, cn, _lib.ptr(buf), _lib.ptr(wsp), wsp.numel(),
-                                               C.c_void_p(st.cuda_stream)), 'gims_gaussian_pyramid')
-    return DevicePyramid(buf, d_off, d_h, d_w, shapes, offs, cn, up[img_at:])
+            wsp = torch.empty(int(L.gims_pyramid_workspace_bytes(h, w, cn)), dtype=torch.uint8, device=dev)
+            _lib.check(L.gims_gaussian_pyramid(_lib.ptr(d_img), h, w, cn, _lib.ptr(buf), _lib.ptr(wsp), wsp.numel(),
+                                               C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)),
+                       'gims_gaussian_pyramid')
+    return DevicePyramid(buf, d_off, d_h, d_w, shapes, offs, cn, d_img)
 
 
 def extract_patches_device(kps, levels, device):
     """`extract_patches` on the GPU: (N, 32, 32[, C]) float32 ON `device`, bit-identical to the host path (the kernel follows
     OpenCV's 8-bit fixed-point cubic warp, csrc/patches.cu).  `levels`: the host pyramid (a list of uint8 arrays; the
     levels that carry keypoints are uploaded) or a `DevicePyramid` of the same device (nothing is uploaded).  `kps`: a list
-    of cv2.KeyPoint or the `DeviceKeypoints` of `detect_device`."""
-    import ctypes as C
-    from . import _lib
+    of cv2.KeyPoint or the `DeviceKeypoints` of `detect_device`.  A keypoint whose level is not in the pyramid raises
+    GimsError."""
     dev = torch.device(device)
     if dev.type != 'cuda':
         raise _lib.GimsError('extract_patches_device needs a CUDA device')
     n = len(kps)
-    on_device = isinstance(levels, DevicePyramid)
-    if on_device:
+    if isinstance(levels, DevicePyramid):
         pdev = levels.buffer.device
         if dev.index is not None and dev.index != pdev.index:
             raise _lib.GimsError('extract_patches_device: the pyramid is on %s, not %s' % (pdev, dev))
@@ -306,49 +318,38 @@ def extract_patches_device(kps, levels, device):
     if n == 0:
         return out
     level, inv = patch_maps_from_arrays(*kps.host()) if isinstance(kps, DeviceKeypoints) else patch_maps(kps)
-    st = torch.cuda.current_stream(dev)
-    if on_device:
-        if int(level.max()) >= len(levels):
-            raise _lib.GimsError('extract_patches_device: a keypoint names level %d of a %d-level pyramid'
-                                 % (int(level.max()), len(levels)))
-        with torch.cuda.device(dev):
-            d_level = torch.from_numpy(level).to(dev)
-            d_inv = torch.from_numpy(inv).to(dev)
-            _lib.check(_lib.lib().gims_extract_patches(_lib.ptr(levels.buffer), _lib.ptr(levels.offset),
-                                                       _lib.ptr(levels.height), _lib.ptr(levels.width), len(levels), cn,
-                                                       _lib.ptr(d_level), _lib.ptr(d_inv), n, _lib.ptr(out),
-                                                       C.c_void_p(st.cuda_stream)), 'gims_extract_patches')
-        return out
-    # only the levels that carry keypoints travel (the coarse octaves are small, the unused fine ones are not)
+    _check_levels(level, len(levels))
+    with torch.cuda.device(dev):
+        if isinstance(levels, DevicePyramid):
+            buf, d_off, d_h, d_w = levels.buffer, levels.offset, levels.height, levels.width
+        else:
+            buf, d_off, d_h, d_w = _upload_host_levels(levels, level, dev)
+        d_level = torch.from_numpy(level).to(dev)
+        d_inv = torch.from_numpy(inv).to(dev)
+        _lib.check(_lib.lib().gims_extract_patches(_lib.ptr(buf), _lib.ptr(d_off), _lib.ptr(d_h), _lib.ptr(d_w),
+                                                   len(levels), cn, _lib.ptr(d_level), _lib.ptr(d_inv), n, _lib.ptr(out),
+                                                   C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)),
+                   'gims_extract_patches')
+    return out
+
+
+def _upload_host_levels(levels, level, dev):
+    """The levels of a host pyramid that `level` names, with the level table of the whole pyramid, as
+    `_upload_level_table` returns them; only those levels travel (the coarse octaves are small, the unused fine ones are
+    not)."""
     used = np.zeros(len(levels), dtype=bool)
     used[level] = True
     sizes = [int(l.size) if u else 0 for l, u in zip(levels, used)]
     offs = np.concatenate([[0], np.cumsum(sizes)[:-1]]).astype(np.int64)
-    total = int(sum(sizes))
-    flat = _pinned_staging(total)
-    fl = flat.numpy()
+    parts = []
     for l, o, u in zip(levels, offs, used):
-        if not u:
-            continue
-        if l.dtype != np.uint8:
-            raise _lib.GimsError('extract_patches_device: pyramid levels must be uint8 (got %s)' % l.dtype)
-        np.copyto(fl[o:o + l.size].reshape(l.shape), l)
-    with torch.cuda.device(dev):
-        d_lv = flat[:total].to(dev, non_blocking=True)
-        _STAGING.event = torch.cuda.Event()
-        _STAGING.event.record(st)                 # the staging buffer is reused by this thread's next call
-        d_off = torch.from_numpy(offs).to(dev)
-        d_h = torch.tensor([l.shape[0] for l in levels], dtype=torch.int32, device=dev)
-        d_w = torch.tensor([l.shape[1] for l in levels], dtype=torch.int32, device=dev)
-        d_level = torch.from_numpy(level).to(dev)
-        d_inv = torch.from_numpy(inv).to(dev)
-        _lib.check(_lib.lib().gims_extract_patches(_lib.ptr(d_lv), _lib.ptr(d_off), _lib.ptr(d_h), _lib.ptr(d_w), len(levels), cn,
-                                                   _lib.ptr(d_level), _lib.ptr(d_inv), n, _lib.ptr(out),
-                                                   C.c_void_p(st.cuda_stream)), 'gims_extract_patches')
-        # the staging buffers may be freed once the stream has passed this point
-        for t in (d_lv, d_off, d_h, d_w, d_level, d_inv):
-            t.record_stream(st)
-    return out
+        if u:
+            if l.dtype != np.uint8:
+                raise _lib.GimsError('extract_patches_device: pyramid levels must be uint8 (got %s)' % l.dtype)
+            parts.append((int(o), l))
+    hs = np.array([l.shape[0] for l in levels], dtype=np.int32)
+    ws = np.array([l.shape[1] for l in levels], dtype=np.int32)
+    return _upload_level_table(offs, hs, ws, parts, int(sum(sizes)), dev)
 
 
 def describe(patches, carhynet, device, batch_size=512):
@@ -380,41 +381,7 @@ def describe(patches, carhynet, device, batch_size=512):
     return d.to(device)
 
 
-def device_pyramids(images, device):
-    """Enqueue `gaussian_pyramid_device` for every image of `images` that it takes (uint8, 1 or 3 channels) when `device`
-    is a CUDA device and GIMS_HOST_PATCHES is not 1; None for the others, whose pyramid stays on the host."""
-    on_gpu = torch.device(device).type == 'cuda' and os.environ.get('GIMS_HOST_PATCHES') != '1'
-    return [gaussian_pyramid_device(img, device) if on_gpu and pyramid_on_device(img) else None for img in images]
-
-
-def host_stages(image_sets, max_kp=-1, pyramids=None):
-    """The OpenCV stages (SIFT detection + Gaussian pyramid) of several images side by side — OpenCV releases the GIL, and
-    the reference runs image 0 and image 1 one after the other (matching.py:18-24).  `image_sets`: a list of iterables of
-    images (each what `data['image']` is); returns, per set, a list of (keypoints, pyramid levels).  `pyramids`, if given,
-    holds per set and image a pyramid already built (a `DevicePyramid`) or None: only the None ones are built here."""
-    flat = [np.asarray(img) for imgs in image_sets for img in imgs]
-    counts = [len(imgs) for imgs in image_sets]
-    pyrs = [p for ps in pyramids for p in ps] if pyramids is not None else [None] * len(flat)
-
-    def stage(args):
-        img, pyr = args
-        return detect(img, max_kp), (gaussian_pyramid(img) if pyr is None else pyr)
-    if len(flat) > 1:
-        from concurrent.futures import ThreadPoolExecutor
-        with ThreadPoolExecutor(max_workers=min(len(flat), 8)) as pool:
-            done = list(pool.map(stage, zip(flat, pyrs)))
-    else:
-        done = [stage(a) for a in zip(flat, pyrs)]
-    out, i = [], 0
-    for c in counts:
-        out.append(done[i:i + c])
-        i += c
-    return out
-
-
 SIFT_KP_CAP = 16384             # first keypoint capacity of detect_device; 4x more on each overflow
-_SIFT_WS = {}                   # (device, stream, thread) -> grow-only uint8 workspace of gims_sift_detect
-_SIFT_WS_LOCK = __import__('threading').Lock()
 
 
 class DeviceKeypoints:
@@ -445,8 +412,6 @@ class _PendingDetect:
     """A detection enqueued by `detect_enqueue`: the device outputs and their pinned host copy, not yet waited for."""
 
     def __init__(self, image, h, w, cn, dev, max_keypoints, kp_cap):
-        import ctypes as C
-        from . import _lib
         self.args = (image, h, w, cn, dev, max_keypoints)
         self.cap = kp_cap
         L = _lib.lib()
@@ -458,14 +423,7 @@ class _PendingDetect:
             self.pt = f[4:4 + 2 * kp_cap].view(kp_cap, 2)
             self.size, self.angle, self.response = (f[4 + k * kp_cap:4 + (k + 1) * kp_cap] for k in (2, 3, 4))
             self.octave = out[4 + 5 * kp_cap:]
-            need = int(L.gims_sift_workspace_bytes(h, w, cn, kp_cap))
-            key = (str(dev), st.cuda_stream, __import__('threading').get_ident())
-            with _SIFT_WS_LOCK:
-                wsp = _SIFT_WS.get(key)
-            if wsp is None or wsp.numel() < need:
-                wsp = torch.empty(need, dtype=torch.uint8, device=dev)
-                with _SIFT_WS_LOCK:
-                    _SIFT_WS[key] = wsp
+            wsp = torch.empty(int(L.gims_sift_workspace_bytes(h, w, cn, kp_cap)), dtype=torch.uint8, device=dev)
             _lib.check(L.gims_sift_detect(_lib.ptr(image), h, w, cn, max_keypoints, kp_cap, _lib.ptr(wsp), wsp.numel(),
                                           _lib.ptr(self.pt), _lib.ptr(self.size), _lib.ptr(self.angle),
                                           _lib.ptr(self.response), _lib.ptr(self.octave), _lib.ptr(out[0:1]),
@@ -478,7 +436,6 @@ class _PendingDetect:
 
     def result(self):
         """Wait for the read-back; on GIMS_STATUS_KEYPOINT_OVERFLOW run again with 4x the capacity."""
-        from . import _lib
         self.done.synchronize()
         hv = self.host.numpy()
         status = int(hv[1])
@@ -497,20 +454,14 @@ def detect_enqueue(image, device, max_keypoints=-1, pyramid=None, kp_cap=SIFT_KP
     """Enqueue `detect_device` on the current stream of `device` without waiting; `.result()` of the returned object
     waits and gives the `DeviceKeypoints`.  `pyramid`: the `DevicePyramid` of the same image, whose uploaded copy is
     reused (otherwise the image is uploaded here)."""
-    from . import _lib
+    img, h, w, cn = _device_image(image, device, 'detect_device')
     dev = torch.device(device)
-    if dev.type != 'cuda':
-        raise _lib.GimsError('detect_device needs a CUDA device')
-    img = np.asarray(image)
-    if not pyramid_on_device(img):
-        raise _lib.GimsError('detect_device: need a uint8 (H, W), (H, W, 1) or (H, W, 3) image (got %s %s)'
-                             % (img.dtype, img.shape))
-    h, w = img.shape[:2]
-    cn = 3 if img.ndim == 3 and img.shape[2] == 3 else 1
     if pyramid is not None and pyramid.image is not None:
         d_img = pyramid.image
         dev = d_img.device
     else:
+        # not `_pinned_upload`: its single-threaded copy into the staging buffer made this call 0.1 ms slower per
+        # 800 x 600 colour image on a B200 than torch's own copy into freshly pinned memory
         with torch.cuda.device(dev):
             d_img = torch.from_numpy(np.ascontiguousarray(img).reshape(-1)).pin_memory().to(dev, non_blocking=True)
     return _PendingDetect(d_img, h, w, cn, dev, int(max_keypoints), int(kp_cap))
@@ -524,31 +475,75 @@ def detect_device(image, device, max_keypoints=-1, pyramid=None):
     return detect_enqueue(image, device, max_keypoints, pyramid).result()
 
 
+def _patches_on_device(device):
+    """True if the patches of host levels are cut on `device`: a CUDA device, unless GIMS_HOST_PATCHES=1 keeps the host
+    loop."""
+    return torch.device(device).type == 'cuda' and os.environ.get('GIMS_HOST_PATCHES') != '1'
+
+
+def _use_device_pyramid(image, device, detector):
+    """True if `stage_images` builds this image's pyramid on the device: always for the device detector, which reads the
+    image the pyramid uploads; for cv2's, when the patches are cut on the device and the kernel takes the image."""
+    return detector == 'device' or (_patches_on_device(device) and pyramid_on_device(image))
+
+
+def stage_images(image_sets, device, max_keypoints=-1, detector='opencv'):
+    """Keypoints and pyramids of several images: `image_sets` is a list of iterables of images (each what `data['image']`
+    is); returns, per set and image, (keypoints, levels).  The device pyramids are enqueued first, on the current stream
+    of `device`, so that they run while the host works.  With `detector='device'` the detection of every image is
+    enqueued next and then waited for: the keypoints are `DeviceKeypoints`, the levels a `DevicePyramid`.  With
+    'opencv', cv2 detection, and the host pyramid of an image without a device one, run for all images side by side
+    (OpenCV releases the GIL; the reference runs image 0, then image 1, matching.py:18-24): the keypoints are lists of
+    cv2.KeyPoint, the levels a `DevicePyramid` or a list of host arrays."""
+    sets = [[np.asarray(img) for img in imgs] for imgs in image_sets]
+    flat = [img for imgs in sets for img in imgs]
+    pyrs = [gaussian_pyramid_device(img, device) if _use_device_pyramid(img, device, detector) else None for img in flat]
+    if detector == 'device':
+        pending = [detect_enqueue(img, device, max_keypoints, pyramid=pyr) for img, pyr in zip(flat, pyrs)]
+        done = [(p.result(), pyr) for p, pyr in zip(pending, pyrs)]
+    else:
+        def stage(args):
+            img, pyr = args
+            return detect(img, max_keypoints), (gaussian_pyramid(img) if pyr is None else pyr)
+        if len(flat) > 1:
+            with ThreadPoolExecutor(max_workers=min(len(flat), 8)) as pool:
+                done = list(pool.map(stage, zip(flat, pyrs)))
+        else:
+            done = [stage(a) for a in zip(flat, pyrs)]
+    out, i = [], 0
+    for imgs in sets:
+        out.append(done[i:i + len(imgs)])
+        i += len(imgs)
+    return out
+
+
+def _points_and_scores(kps, device):
+    """(N, 2) pixel xy and (N,) responses, float32 on `device`, of a list of cv2.KeyPoint or of `DeviceKeypoints`."""
+    if isinstance(kps, DeviceKeypoints):
+        return kps.pt, kps.response
+    pts = np.array([k.pt for k in kps], dtype=np.float32).reshape(-1, 2)
+    resp = np.array([k.response for k in kps], dtype=np.float32)
+    return torch.from_numpy(pts).to(device), torch.from_numpy(resp).to(device)
+
+
 def sift_forward(data, device, staged=None):
     """Same dict in / dict out as utils/common.py:837-893: `data['image']` iterates over images, `data['carhynet']` is the
     caller's descriptor object; returns lists (one entry per image) of device tensors
     `keypoints` (N, 2) fp32 pixel xy, `scores` (N,) fp32 SIFT responses, `descriptors` (256, N) fp32.
-    `staged`: the (keypoints, pyramid) pairs of the images if `host_stages` has already produced them.  On a CUDA device
-    the pyramid of a uint8 grey or colour image is built there (enqueued before detection starts, so the two overlap)."""
-    max_kp = data.get('max_keypoints', -1)
-    kpts, scores, descs = [], [], []
-    images = [np.asarray(img) for img in data['image']]
+    `staged`: the (keypoints, levels) pairs of the images if `stage_images` has already produced them; otherwise it runs
+    here with cv2's detector.  The patches are cut on the device from a `DevicePyramid`, and from host levels unless
+    `_patches_on_device` says otherwise."""
     if staged is None:
-        staged = host_stages([images], max_kp, [device_pyramids(images, device)])[0]
-    for img, (kps, levels) in zip(images, staged):
-        if isinstance(levels, DevicePyramid):
+        staged = stage_images([data['image']], device, data.get('max_keypoints', -1))[0]
+    kpts, scores, descs = [], [], []
+    for kps, levels in staged:
+        if isinstance(levels, DevicePyramid) or _patches_on_device(device):
             patches = extract_patches_device(kps, levels, device)
         else:
-            on_gpu = torch.device(device).type == 'cuda' and levels[0].dtype == np.uint8 and os.environ.get('GIMS_HOST_PATCHES') != '1'
-            patches = extract_patches_device(kps, levels, device) if on_gpu else extract_patches(kps, levels)
+            patches = extract_patches(kps, levels)
         d = describe(patches, data['carhynet'], device)                        # (N, 128), on the device
-        if isinstance(kps, DeviceKeypoints):
-            kpts.append(kps.pt)
-            scores.append(kps.response)
-        else:
-            pts = np.array([k.pt for k in kps], dtype=np.float32).reshape(-1, 2)
-            resp = np.array([k.response for k in kps], dtype=np.float32)
-            kpts.append(torch.from_numpy(pts).to(device))
-            scores.append(torch.from_numpy(resp).to(device))
+        pt, score = _points_and_scores(kps, device)
+        kpts.append(pt)
+        scores.append(score)
         descs.append(torch.cat([d, d], dim=1).t().contiguous())                # utils/common.py:891
     return {'keypoints': kpts, 'scores': scores, 'descriptors': descs}

@@ -1,9 +1,7 @@
 """Host-side mirror of the reference's `Matching` front-end (models/matching.py:8-30)."""
-import numpy as np
 import torch
 
-from . import _lib
-from .frontend import detect_enqueue, device_pyramids, gaussian_pyramid_device, host_stages, sift_forward
+from .frontend import sift_forward, stage_images
 from .gmatcher import GMatcher
 
 
@@ -30,34 +28,16 @@ class Matching(torch.nn.Module):
         self.gmodel = GMatcher(config)
         self.max_keypoints = config.get('max_keypoints', -1)
 
-    def _device_stages(self, images, dev):
-        """Pyramid and detection of every image enqueued on the device, then one wait: per set, (keypoints, pyramid)."""
-        if torch.device(dev).type != 'cuda':
-            raise _lib.GimsError("Matching: 'detector': 'device' needs a CUDA device (got %s)" % dev)
-        pending = []
-        for imgs in images:
-            row = []
-            for img in imgs:
-                pyr = gaussian_pyramid_device(img, dev)
-                row.append((detect_enqueue(img, dev, self.max_keypoints, pyramid=pyr), pyr))
-            pending.append(row)
-        return [[(p.result(), pyr) for p, pyr in row] for row in pending]
-
     def forward(self, data):
         pred = {}
         need = [s for s in ('0', '1') if 'keypoints' + s not in data]
         dev = data.get('device', self.gmodel.bin_score.device)
-        # the pyramids go onto the caller's stream first (uint8 grey / colour images, CUDA device); the OpenCV stages of
-        # both images then run side by side (the reference does image 0, then image 1)
-        images = [[np.asarray(img) for img in data['image' + s]] for s in need]
-        if self.detector == 'device':
-            staged = dict(zip(need, self._device_stages(images, dev)))
-        else:
-            pyramids = [device_pyramids(imgs, dev) for imgs in images]
-            staged = dict(zip(need, host_stages(images, self.max_keypoints, pyramids))) if need else {}
-        for s in need:
+        # both images are staged at once: the device work of both is enqueued first, then the host work of the two runs
+        # side by side (the reference does image 0, then image 1)
+        staged = stage_images([data['image' + s] for s in need], dev, self.max_keypoints, self.detector) if need else []
+        for s, st in zip(need, staged):
             out = sift_forward({'image': data['image' + s], 'max_keypoints': self.max_keypoints,
-                                'carhynet': data['carhynet']}, device=dev, staged=staged[s])
+                                'carhynet': data['carhynet']}, device=dev, staged=st)
             pred = {**pred, **{k + s: v for k, v in out.items()}}
         data = {**data, **pred}
         for k in data:

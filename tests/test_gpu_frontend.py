@@ -53,3 +53,21 @@ def test_sift_forward_device_patches_equal_host_patches(monkeypatch):
     assert torch.equal(got['keypoints'][0], want['keypoints'][0])
     assert got['descriptors'][0].shape == (256, 500)
     assert torch.allclose(got['descriptors'][0], want['descriptors'][0], atol=1e-6)
+
+
+def test_keypoint_outside_the_pyramid_raises():
+    from gims_b200 import _lib
+    from gims_b200 import frontend as fe
+    from gims_b200.synth import make_textured_image
+    img = make_textured_image(240, 320, seed=3)
+    kps = fe.detect(img, 50)
+    host = fe.gaussian_pyramid(img)
+    sources = {'host levels': host, 'device pyramid': fe.gaussian_pyramid_device(img, 'cuda:0')}
+    past = len(host) // (fe.LAYERS + 3) - 1                   # the octave after the coarsest one: level len(host)
+    for octave in (0xFE, past):                               # 0xFE unpacks to octave -2: level -6
+        bad = kps + [cv2.KeyPoint(100, 100, 8, 0, 1, octave)]
+        for name, levels in sources.items():
+            with pytest.raises(_lib.GimsError, match='level'):
+                fe.extract_patches_device(bad, levels, 'cuda:0')
+    for name, levels in sources.items():                     # the good keypoints still go through
+        assert fe.extract_patches_device(kps, levels, 'cuda:0').shape[0] == len(kps), name

@@ -96,7 +96,7 @@ def _call(matching, car, pair, dev):
     return {k: v[0].cpu() for k, v in pred.items()}
 
 
-def test_matching_with_images_equals_host_pyramid_route(monkeypatch):
+def test_matching_with_images_equals_forced_host_pyramid_route(monkeypatch):
     dev = torch.device('cuda:0')
     monkeypatch.setattr(torch.backends.cudnn, 'deterministic', True)
     monkeypatch.setattr(torch.backends.cudnn, 'benchmark', False)
@@ -105,9 +105,7 @@ def test_matching_with_images_equals_host_pyramid_route(monkeypatch):
     got = _call(matching, car, pair, dev)
     from gims_b200 import frontend as fe
     # the old route: host pyramid, levels uploaded by extract_patches_device
-    monkeypatch.setattr(fe, 'device_pyramids', lambda images, device: [None] * len(images))
-    import gims_b200.matching as gm
-    monkeypatch.setattr(gm, 'device_pyramids', lambda images, device: [None] * len(images))
+    monkeypatch.setattr(fe, '_use_device_pyramid', lambda image, device, detector: False)
     want = _call(matching, car, pair, dev)
     for s in '01':
         assert torch.equal(got['keypoints' + s], want['keypoints' + s])

@@ -63,3 +63,17 @@ def test_patch_maps_equal_per_keypoint_construction():
         affine = np.hstack([rot, [[r - shift[0]], [r - shift[1]]]])
         assert level[i] == (octave - fe.FIRST_OCTAVE) * (fe.LAYERS + 3) + layer
         assert np.allclose(inv[i], cw.invert_affine(affine), rtol=1e-15, atol=0)
+
+
+def test_level_check_rejects_keypoints_outside_the_pyramid():
+    from gims_b200 import _lib
+    from gims_b200 import frontend as fe
+    n_levels = 8 * (fe.LAYERS + 3)
+    inside = [cv2.KeyPoint(10, 10, 4, 0, 1, o) for o in (0xFF, 0x500 | 6)]     # level 0, the last level
+    fe._check_levels(fe.patch_maps(inside)[0], n_levels)
+    below = cv2.KeyPoint(10, 10, 4, 0, 1, 0xFE)                                  # octave -2: level -6
+    past = cv2.KeyPoint(10, 10, 4, 0, 1, 7)                                      # octave 7: level 48
+    for kp, level in ((below, -6), (past, n_levels)):
+        assert fe.patch_maps([kp])[0][0] == level
+        with pytest.raises(_lib.GimsError, match='level %d of a %d-level' % (level, n_levels)):
+            fe._check_levels(fe.patch_maps(inside + [kp])[0], n_levels)

@@ -87,7 +87,12 @@ def main():
     # -- the whole image-input call, old route against new, alternated -------------------------------------------------
     def old_route(p):
         """Matching.forward as it was: detection and the host pyramid side by side, levels uploaded per image."""
-        staged = fe.host_stages([p[0], p[1]], args.kpts)
+        device_pyramid = fe._use_device_pyramid
+        fe._use_device_pyramid = lambda image, device, detector: False
+        try:
+            staged = fe.stage_images([p[0], p[1]], dev, args.kpts)
+        finally:
+            fe._use_device_pyramid = device_pyramid
         data = dict(knobs)
         for s, imgs in (('0', p[0]), ('1', p[1])):
             f = fe.sift_forward({'image': imgs, 'max_keypoints': args.kpts, 'carhynet': car}, dev, staged=staged[int(s)])
