@@ -145,6 +145,10 @@ SIGNATURES = {
     'gims_gt_matches': (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_float, C.c_int, C.c_void_p,
                                   C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     'gims_match_counts': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    'gims_homography_workspace_bytes': (C.c_size_t, [C.c_int, C.c_int]),
+    'gims_find_homographies': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_double, C.c_int, C.c_double,
+                                         C.c_ulonglong, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p,
+                                         C.c_void_p, C.c_void_p]),
     'gims_pair_workspace_bytes': (C.c_size_t, [C.c_void_p, C.c_int, C.c_int, C.c_int]),
     'gims_forward_pair': (C.c_int, [C.c_void_p, C.POINTER(PairInputs), C.POINTER(PairOutputs), C.c_void_p,
                                     C.c_size_t, C.c_void_p]),

@@ -154,3 +154,20 @@ def warp_image(img, seed=0):
     h, w = img.shape[:2]
     hmat = _random_homography(torch.Generator().manual_seed(int(seed)), w, h).numpy()
     return cv2.warpPerspective(img, hmat, (w, h)), hmat.astype(np.float32)
+
+
+def make_correspondences(m, inlier_ratio, noise=1.0, seed=0, width=800, height=600):
+    """Matched points of one synthetic pair for the homography estimator: (src, dst) float32 (m, 2) and the true H (3, 3)
+    float64.  round(m * inlier_ratio) matches follow H with Gaussian noise of `noise` px on the destination; the others
+    are uniform over the image on both sides.  The matches are in random order."""
+    import numpy as np
+    hmat = _random_homography(torch.Generator().manual_seed(int(seed)), width, height).numpy()
+    rng = np.random.default_rng(int(seed) + 7919)
+    n_in = int(round(m * inlier_ratio))
+    wh = np.array([width, height], dtype=np.float64)
+    src = rng.random((m, 2)) * wh
+    proj = np.concatenate([src, np.ones((m, 1))], axis=1) @ hmat.T
+    dst = proj[:, :2] / proj[:, 2:] + rng.normal(0.0, noise, (m, 2))
+    dst[n_in:] = rng.random((m - n_in, 2)) * wh
+    perm = rng.permutation(m)
+    return src[perm].astype(np.float32), dst[perm].astype(np.float32), hmat

@@ -302,6 +302,26 @@ GIMS_API int gims_gt_matches(const float* kpts0, int n0, const float* kpts1, int
 GIMS_API int gims_match_counts(const int64_t* matches0, const int* gt0, int n0_max, const int* n_dev /* may be NULL */,
                       int* counts_dev, void* stream);
 
+/* ---- RANSAC homographies of a batch of matched point sets ---------------------------------------------------------
+ * gims_find_homographies replaces cv2.findHomography(mkpts0, mkpts1, cv2.RANSAC, thresh) of eval_homography.py:180-235
+ * (the homography behind the AUC) and eval_matches.py (the inlier count), for n_pairs pairs in one call.  The algorithm is the
+ * deterministic restatement oracle/ransac_oracle.py fixes (cv2's RANSAC + DLT + Levenberg-Marquardt refinement, with a
+ * counter-based sampler and Gaussian-elimination solves); the results equal it bit for bit, and a pair gives the same
+ * result alone and in any batch.
+ *   src, dst: [total][2] fp32 pixel xy on the device; pair p owns rows [offsets_dev[p], offsets_dev[p+1]) (device int32
+ *   [n_pairs + 1], non-decreasing, from 0).  thresh: reprojection threshold in pixels (> 0); max_iters >= 1 hypotheses;
+ *   0 < confidence < 1; seed: the sampler's key.
+ *   H_out [n_pairs][9] fp64 row-major with H[8] = 1; mask_out [total] uint8, 1 for the inliers of H; n_inliers [n_pairs];
+ *   n_iters [n_pairs] the number of hypotheses run (may be NULL).  "Not found" (fewer than 4 points, a degenerate set,
+ *   or no hypothesis with more than 3 inliers) is n_inliers = 0, H = 0 and a zero mask.  Pairs with 4 points get the
+ *   DLT of the four and an all-ones mask, as in cv2.
+ *   Enqueue-only on `stream`; the workspace holds gims_homography_workspace_bytes(n_pairs, offsets_dev[n_pairs]). */
+GIMS_API size_t gims_homography_workspace_bytes(int n_pairs, int total_points);
+GIMS_API int gims_find_homographies(const float* src, const float* dst, const int* offsets_dev, int n_pairs, double thresh,
+                           int max_iters, double confidence, unsigned long long seed, void* workspace,
+                           size_t workspace_bytes, double* H_out, unsigned char* mask_out, int* n_inliers, int* n_iters,
+                           void* stream);
+
 /* ---- whole pair: replaces GMatcher.forward (gmatcher.py:219-307), test mode ----------------- */
 typedef struct {
   const float* kpts[2];          /* [n][2] */
