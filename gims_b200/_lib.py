@@ -9,13 +9,14 @@ from .build import LIB_PATH
 
 MAX_LAYERS = 64
 MAX_KENC = 8
-MAX_KPTS = 16384
+MAX_KPTS = 65536
 MAX_BATCH = 4
 STATUS_EDGE_OVERFLOW = 1
 STATUS_SINKHORN_TIMEOUT = 2
 STATUS_ERROR_MASK = 0xff
 STATUS_SINKHORN_FAST = 0x100
 STATUS_SINKHORN_EXACT = 0x200
+STATUS_SINKHORN_WIDE = 0x400
 GEMM_SIMT, GEMM_TC, GEMM_TC_F16, GEMM_BF16 = 0, 1, 2, 3
 GEMM_MODES = {'simt': GEMM_SIMT, 'tf32': GEMM_TC, 'tc': GEMM_TC, 'f16': GEMM_TC_F16, 'bf16': GEMM_BF16}
 STATUS_FP16_RANGE = 4

@@ -413,12 +413,12 @@ __global__ void __launch_bounds__(256) k_iso_nn(const float2* __restrict__ kpts,
 __global__ void __launch_bounds__(1024) k_iso_resolve(int n, const int* __restrict__ deg, const int* __restrict__ n_base_edges,
                                                       const int* __restrict__ nn, int* __restrict__ iso_u, int* __restrict__ iso_v,
                                                       int* __restrict__ iso_count, int* __restrict__ extra_cnt) {
-  __shared__ unsigned char hit[GIMS_MAX_KPTS];
+  __shared__ unsigned hit[GIMS_MAX_KPTS / 32];   // one bit per node (8 KB at 65536 nodes)
   __shared__ int warp_tot[32];
   __shared__ int carry_s;
   if (*n_base_edges == 0) return;   // agc.py:487: graphs without edges are returned untouched
   int t = threadIdx.x, lane = t & 31, wid = t >> 5;
-  for (int i = t; i < n; i += 1024) hit[i] = 0;
+  for (int i = t; i < (n + 31) / 32; i += 1024) hit[i] = 0u;
   if (t == 0) carry_s = 0;
   __syncthreads();
   // compaction: iso_u[k] = k-th isolated node (ascending), iso_v[k] = its nearest neighbour (tentative)
@@ -457,10 +457,10 @@ __global__ void __launch_bounds__(1024) k_iso_resolve(int n, const int* __restri
     for (int s = 0; s < m; ++s) {
       int su = __shfl_sync(0xffffffffu, u, s);
       int sv = __shfl_sync(0xffffffffu, v, s);
-      int h = hit[su];                      // all lanes read the same byte
+      const unsigned h = (hit[su >> 5] >> (su & 31)) & 1u;   // all lanes read the same word
       if (!h) {
         active |= 1u << s;
-        if (lane == 0) { hit[sv] = 1; hit[su] = 1; }
+        if (lane == 0) { hit[sv >> 5] |= 1u << (sv & 31); hit[su >> 5] |= 1u << (su & 31); }
       }
       __syncwarp();
     }
@@ -481,39 +481,47 @@ __global__ void __launch_bounds__(1024) k_iso_resolve(int n, const int* __restri
 // ---------------------------------------------------------------------------------------------
 // a-4  connected components: lock-free union-find, smaller root wins (root == smallest member id)
 // ---------------------------------------------------------------------------------------------
-// The whole component search in ONE CTA with the parent array in SHARED memory (n <= 16384 nodes = 64 KB): a find is a
-// chain of dependent loads, and through L2 (volatile, ~500 clk per hop) the grid-wide version took 40-86 us for 15 k edges
-// however the unions were distributed; in shared memory a hop is ~30 clk.  Init, base-graph unions, isolated-node unions
-// and the final labelling are one launch instead of four.
+// The whole component search in ONE CTA with the parent array in SHARED memory: a find is a chain of dependent loads, and
+// through L2 (volatile, ~500 clk per hop) the grid-wide version took 40-86 us for 15 k edges however the unions were
+// distributed; in shared memory a hop is ~30 clk.  Init, base-graph unions, isolated-node unions and the final labelling
+// are one launch instead of four.  Parents are `int` up to 16384 nodes (64 KB) and `unsigned short` above: every node id
+// is below GIMS_MAX_KPTS = 65536, so 16 bits hold it and 65536 nodes take 128 KB (16-bit atomicCAS exists since sm_70).
 //   init: every node points at its smallest neighbour if that is smaller than itself (CSR rows are ascending, so it is the
 //   first entry) — pointers only ever go to strictly smaller ids along real edges, a forest with the same components;
-//   union: lock-free, smaller root wins (root == smallest member id whatever the order of the unions).
-__device__ __forceinline__ int ufs_find(volatile int* p, int x) {
+//   union: lock-free, smaller root wins (root == smallest member id whatever the order of the unions), so the labels do
+//   not depend on the parent type or on the order of the unions.
+constexpr int kCcIntMaxNodes = 16384;
+static_assert(GIMS_MAX_KPTS <= 65536, "16-bit union-find parents need node ids below 65536");
+template <typename P>
+__device__ __forceinline__ int ufs_find(volatile P* p, int x) {
   int cur = x, par = p[cur];
   while (par != cur) {
     const int gp = p[par];
-    if (gp != par) p[cur] = gp;   // path halving; only ever rewires non-roots to an ancestor
+    if (gp != par) p[cur] = (P)gp;   // path halving; only ever rewires non-roots to an ancestor
     cur = par;
     par = gp;
   }
   return cur;
 }
-__device__ __forceinline__ void ufs_union(int* parent, int a, int b) {
+template <typename P>
+__device__ __forceinline__ void ufs_union(P* parent, int a, int b) {
   while (true) {
-    a = ufs_find(parent, a);
-    b = ufs_find(parent, b);
+    a = ufs_find<P>(parent, a);
+    b = ufs_find<P>(parent, b);
     if (a == b) return;
     if (a > b) { const int t = a; a = b; b = t; }
-    if (atomicCAS(&parent[b], b, a) == b) return;
+    if ((int)atomicCAS(&parent[b], (P)b, (P)a) == b) return;
   }
 }
+template <typename P>
 __global__ void __launch_bounds__(1024) k_cc_components(int* __restrict__ parent_out, int n, const int* __restrict__ indptr,
                                                         const int* __restrict__ idx, int edge_cap, const int* __restrict__ iso_u,
                                                         const int* __restrict__ iso_v, const int* __restrict__ iso_count) {
-  extern __shared__ int sp[];
+  extern __shared__ __align__(16) unsigned char sp_raw[];
+  P* sp = reinterpret_cast<P*>(sp_raw);
   for (int i = threadIdx.x; i < n; i += blockDim.x) {
     const int e0 = indptr[i];
-    sp[i] = (e0 < indptr[i + 1] && e0 < edge_cap) ? min(i, idx[e0]) : i;
+    sp[i] = (P)((e0 < indptr[i + 1] && e0 < edge_cap) ? min(i, idx[e0]) : i);
   }
   __syncthreads();
   // a thread per node (each undirected edge once, from its smaller end): with ~7 edges per node a warp per node leaves
@@ -522,17 +530,29 @@ __global__ void __launch_bounds__(1024) k_cc_components(int* __restrict__ parent
     const int e0 = indptr[i], e1 = min(indptr[i + 1], edge_cap);
     for (int e = e0; e < e1; ++e) {
       const int j = idx[e];
-      if (j > i) ufs_union(sp, i, j);
+      if (j > i) ufs_union<P>(sp, i, j);
     }
   }
   const int n_iso = *iso_count;
-  for (int k = threadIdx.x; k < n_iso; k += blockDim.x) ufs_union(sp, iso_u[k], iso_v[k]);
+  for (int k = threadIdx.x; k < n_iso; k += blockDim.x) ufs_union<P>(sp, iso_u[k], iso_v[k]);
   __syncthreads();
   for (int i = threadIdx.x; i < n; i += blockDim.x) {
     int r = i;
-    while (sp[r] != r) r = sp[r];
+    while ((int)sp[r] != r) r = sp[r];
     parent_out[i] = r;
   }
+}
+
+// The attribute belongs to the function, not to one launch: it is always the most the instantiation can need, so that
+// concurrent callers with different node counts cannot lower it under one another's launch.
+template <typename P>
+int launch_cc_components(const AgcWs& w, int n, int edge_cap, cudaStream_t st) {
+  constexpr int kMaxSmem = (sizeof(P) == sizeof(int) ? kCcIntMaxNodes : GIMS_MAX_KPTS) * (int)sizeof(P);
+  const size_t smem = (size_t)n * sizeof(P);
+  GIMS_CUDA_OK(cudaFuncSetAttribute(k_cc_components<P>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem));
+  k_cc_components<P><<<1, 1024, smem, st>>>(w.parent, n, w.indptr_base, w.idx_base, edge_cap, w.iso_u, w.iso_v, w.iso_count);
+  GIMS_LAUNCH_OK();
+  return GIMS_OK;
 }
 
 __global__ void k_cc_count(const int* __restrict__ label, int n, int* comp_size) {
@@ -876,10 +896,8 @@ extern "C" int gims_agc_build(const float* kpts, const float* desc, int desc_cha
   k_iso_resolve<<<1, 1024, 0, st>>>(n, w.deg_base, n_base_edges, w.nn_iso, w.iso_u, w.iso_v, w.iso_count, w.extra_cnt);
   GIMS_LAUNCH_OK();
   // a-4
-  GIMS_CUDA_OK(cudaFuncSetAttribute(k_cc_components, cudaFuncAttributeMaxDynamicSharedMemorySize, GIMS_MAX_KPTS * (int)sizeof(int)));
-  k_cc_components<<<1, 1024, (size_t)n * sizeof(int), st>>>(w.parent, n, w.indptr_base, w.idx_base, edge_cap, w.iso_u, w.iso_v,
-                                                           w.iso_count);
-  GIMS_LAUNCH_OK();
+  GIMS_TRY(n <= kCcIntMaxNodes ? launch_cc_components<int>(w, n, edge_cap, st)
+                                : launch_cc_components<unsigned short>(w, n, edge_cap, st));
   k_cc_count<<<cdiv(n, 256), 256, 0, st>>>(w.parent, n, w.comp_size);
   GIMS_LAUNCH_OK();
   k_keep_compact<<<1, 1024, 0, st>>>(n, w.parent, w.comp_size, min_size, w.new_id, kept_idx, w.comp_of_root, w.comp_root,

@@ -469,10 +469,6 @@ int validate_pair(const gims_pair_inputs* in, const gims_pair_outputs* o) {
     set_error("gims_forward_pair: keypoint counts (%d, %d) outside [2, %d]", n0, n1, GIMS_MAX_KPTS);
     return GIMS_ERR_ARG;
   }
-  if (n1 > gims_sinkhorn_max_columns()) {
-    set_error("gims_forward_pair: n1=%d exceeds the Sinkhorn kernel's shared-memory limit of %d columns", n1, gims_sinkhorn_max_columns());
-    return GIMS_ERR_ARG;
-  }
   if (in->edge_cap < 1) { set_error("gims_forward_pair: edge_cap %d", in->edge_cap); return GIMS_ERR_ARG; }
   if (!o->n_kept_dev || !o->n_edges_dev || !o->n_comp_dev || !o->thr_dev || !o->mdesc || !o->u || !o->v || !o->status_dev) {
     set_error("gims_forward_pair: null output pointer");

@@ -1109,6 +1109,276 @@ __global__ void k_match_finalize(int n0_max, int n1_max, const int* __restrict__
   }
 }
 
+// =====================================================================================================================
+// Wide iteration: problems whose potentials do not fit shared memory (plan() below rejects them; on a B200 about 56 k
+// columns and more).  The reference's log-sum-exp iteration in the log domain, streamed from global memory with ordinary,
+// non-cooperative launches — three per iteration:
+//   k_wide_rows      u_r = log_mu_r - LSE_j (z_rj + v_j): a CTA per kWideRows rows, v read through L1 / L2;
+//   k_wide_cols      per (row block, column): the (max, sum) partial of LSE_r (z_rj + u_r) over the block's rows;
+//   k_wide_combine   v_j = log_nu_j - LSE over the kWideBlocks partials of column j, merged in row-block order.
+// No float atomics and no grid-wide waits: the results do not change from run to run and nothing can time out.  At
+// 65536 x 65536 the matrix (17.2 GB) is read twice per iteration, so the iteration is bound by HBM; the exponentials
+// (one ex2 per element plus one per chunk of four) hide behind the loads.  The final pass (the same three kernels,
+// FINAL = true) evaluates ((Z0 + u) + v) - norm like the shared-memory kernels and feeds k_match_finalize.
+// Element offsets are 64-bit throughout: (n0 + 1) * ld exceeds 2^31 from 46341 keypoints on.
+// =====================================================================================================================
+constexpr int kWideThreads = 256;
+constexpr int kWideRows = 8;                  // rows per CTA of the row pass
+constexpr int kWideChunk = 4;                 // columns per thread and step of the row pass (strided by kWideThreads)
+constexpr int kWideColsPerThread = 4;         // columns per thread of the column pass (strided by kWideThreads)
+constexpr int kWideRowStep = 8;               // rows per step of the column pass
+constexpr int kWideBlocks = kMaxGrid;         // row blocks of the column pass: the partial buffer is the kernels' `part`
+
+struct WideDims {
+  int n0, n1;                                 // live counts
+  float norm, log_mu_last, log_nu_last;
+};
+__device__ __forceinline__ WideDims wide_dims(int n0_max, int n1_max, const int* n_dev) {
+  WideDims d;
+  d.n0 = n_dev ? min(n_dev[0], n0_max) : n0_max;
+  d.n1 = n_dev ? min(n_dev[1], n1_max) : n1_max;
+  const float ms = (float)d.n0, ns = (float)d.n1;          // as sink_geom (gmatcher.py:62-64)
+  d.norm = -logf(ms + ns);
+  d.log_mu_last = logf(ns) + d.norm;
+  d.log_nu_last = logf(ms) + d.norm;
+  return d;
+}
+// rows per block of the column pass over `rows` rows, and the number of blocks that own at least one
+__device__ __forceinline__ int wide_rows_per_block(int rows) { return max(1, (rows + kWideBlocks - 1) / kWideBlocks); }
+
+// (m, s) <- LSE-combine with (pm, ps); empty partials are (-inf, 0) and leave the other side as it is
+__device__ __forceinline__ void lse_merge_safe(float& m, float& s, float pm, float ps) {
+  const float mn = fmaxf(m, pm);
+  if (mn == -CUDART_INF_F) return;
+  s = s * ex2((m - mn) * kLog2e) + ps * ex2((pm - mn) * kLog2e);
+  m = mn;
+}
+// online LSE over a chunk of N values (-inf = masked): one rescale per chunk, one ex2 per value
+template <int N>
+__device__ __forceinline__ void lse_chunk(float& m, float& s, const float* x) {
+  float cm = x[0];
+#pragma unroll
+  for (int k = 1; k < N; ++k) cm = fmaxf(cm, x[k]);
+  const float mn = fmaxf(m, cm);
+  if (mn == -CUDART_INF_F) return;
+  float acc = s * ex2((m - mn) * kLog2e);
+#pragma unroll
+  for (int k = 0; k < N; ++k) acc += ex2((x[k] - mn) * kLog2e);
+  s = acc;
+  m = mn;
+}
+__device__ __forceinline__ bool argmax_better(float b, int j, float best, int bj) { return b > best || (b == best && j < bj); }
+
+// Row pass.  FINAL = false: u_r for the live rows r <= n0 (dustbin row included) from the current v.
+// FINAL = true: row max + first argmax of ((z + u_r) + v_j) - norm over the keypoint columns, rows < n0.
+template <bool FINAL>
+__global__ void __launch_bounds__(kWideThreads) k_wide_rows(const float* __restrict__ Z, size_t ld, int n0_max, int n1_max,
+                                                            const int* __restrict__ n_dev, const float* __restrict__ v,
+                                                            float* __restrict__ u, int* __restrict__ idx0,
+                                                            float* __restrict__ max0) {
+  __shared__ float red_a[kWideThreads / 32][kWideRows];
+  __shared__ float red_b[kWideThreads / 32][kWideRows];
+  const WideDims d = wide_dims(n0_max, n1_max, n_dev);
+  const int rows = FINAL ? d.n0 : d.n0 + 1, cols = FINAL ? d.n1 : d.n1 + 1;
+  const int r0 = blockIdx.x * kWideRows;
+  if (r0 >= rows) return;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  float a[kWideRows], b[kWideRows], ur[kWideRows];        // (max, sum) or (best value, best column as int bits)
+#pragma unroll
+  for (int rr = 0; rr < kWideRows; ++rr) {
+    a[rr] = -CUDART_INF_F;
+    b[rr] = FINAL ? __int_as_float(0x7fffffff) : 0.f;
+    ur[rr] = (FINAL && r0 + rr < rows) ? u[r0 + rr] : 0.f;
+  }
+  const float* zr = Z + (size_t)r0 * ld;
+  for (int j0 = 0; j0 < cols; j0 += kWideChunk * kWideThreads) {
+    float vj[kWideChunk], x[kWideRows][kWideChunk];
+#pragma unroll
+    for (int q = 0; q < kWideChunk; ++q) {
+      const int j = j0 + tid + q * kWideThreads;
+      vj[q] = (j < cols) ? v[j] : 0.f;
+#pragma unroll
+      for (int rr = 0; rr < kWideRows; ++rr)
+        x[rr][q] = (j < cols && r0 + rr < rows) ? __ldcs(zr + (size_t)rr * ld + j) : -CUDART_INF_F;
+    }
+#pragma unroll
+    for (int rr = 0; rr < kWideRows; ++rr) {
+      if (FINAL) {
+#pragma unroll
+        for (int q = 0; q < kWideChunk; ++q) {                // columns ascending: strict > keeps the first maximum
+          const float t = ((x[rr][q] + ur[rr]) + vj[q]) - d.norm;
+          if (t > a[rr]) { a[rr] = t; b[rr] = __int_as_float(j0 + tid + q * kWideThreads); }
+        }
+      } else {
+#pragma unroll
+        for (int q = 0; q < kWideChunk; ++q) x[rr][q] += vj[q];
+        lse_chunk<kWideChunk>(a[rr], b[rr], x[rr]);
+      }
+    }
+  }
+#pragma unroll
+  for (int rr = 0; rr < kWideRows; ++rr) {
+#pragma unroll
+    for (int o = 16; o; o >>= 1) {
+      const float pa = __shfl_xor_sync(0xffffffffu, a[rr], o), pb = __shfl_xor_sync(0xffffffffu, b[rr], o);
+      if (FINAL) {
+        if (argmax_better(pa, __float_as_int(pb), a[rr], __float_as_int(b[rr]))) { a[rr] = pa; b[rr] = pb; }
+      } else {
+        lse_merge_safe(a[rr], b[rr], pa, pb);
+      }
+    }
+    if (lane == 0) { red_a[warp][rr] = a[rr]; red_b[warp][rr] = b[rr]; }
+  }
+  __syncthreads();
+  if (tid < kWideRows && r0 + tid < rows) {
+    const int r = r0 + tid;
+    float m = red_a[0][tid], s = red_b[0][tid];
+    for (int w = 1; w < kWideThreads / 32; ++w) {             // warps in order
+      if (FINAL) {
+        if (argmax_better(red_a[w][tid], __float_as_int(red_b[w][tid]), m, __float_as_int(s))) { m = red_a[w][tid]; s = red_b[w][tid]; }
+      } else {
+        lse_merge_safe(m, s, red_a[w][tid], red_b[w][tid]);
+      }
+    }
+    if (FINAL) {
+      idx0[r] = __float_as_int(s);
+      max0[r] = m;
+    } else {
+      const float lmu = (r == d.n0) ? d.log_mu_last : d.norm;
+      u[r] = lmu - (m + logf(s));
+    }
+  }
+}
+
+// Column pass: CTA (x, y) covers columns [x * 1024, +1024) and row block y.  FINAL = false: (max, sum) of z_rj + u_r over
+// the block's live rows (dustbin row included).  FINAL = true: (best value, first row) of ((z + u_r) + v_j) - norm over
+// the block's keypoint rows, keypoint columns only.
+template <bool FINAL>
+__global__ void __launch_bounds__(kWideThreads) k_wide_cols(const float* __restrict__ Z, size_t ld, int n0_max, int n1_max,
+                                                            const int* __restrict__ n_dev, const float* __restrict__ u,
+                                                            const float* __restrict__ v, float2* __restrict__ part,
+                                                            size_t ldp) {
+  const WideDims d = wide_dims(n0_max, n1_max, n_dev);
+  const int rows = FINAL ? d.n0 : d.n0 + 1, cols = FINAL ? d.n1 : d.n1 + 1;
+  const int rpb = wide_rows_per_block(rows);
+  const int rb = blockIdx.y * rpb, re = min(rb + rpb, rows);
+  const int c0 = blockIdx.x * (kWideColsPerThread * kWideThreads) + threadIdx.x;
+  if (rb >= re || blockIdx.x * (kWideColsPerThread * kWideThreads) >= cols) return;
+  float a[kWideColsPerThread], b[kWideColsPerThread], vj[kWideColsPerThread];
+#pragma unroll
+  for (int q = 0; q < kWideColsPerThread; ++q) {
+    const int j = c0 + q * kWideThreads;
+    a[q] = -CUDART_INF_F;
+    b[q] = FINAL ? __int_as_float(0x7fffffff) : 0.f;
+    vj[q] = (FINAL && j < cols) ? v[j] : 0.f;
+  }
+  for (int r0 = rb; r0 < re; r0 += kWideRowStep) {
+    float x[kWideColsPerThread][kWideRowStep], urs[kWideRowStep];
+#pragma unroll
+    for (int rr = 0; rr < kWideRowStep; ++rr) urs[rr] = (r0 + rr < re) ? u[r0 + rr] : 0.f;
+#pragma unroll
+    for (int q = 0; q < kWideColsPerThread; ++q) {
+      const int j = c0 + q * kWideThreads;
+#pragma unroll
+      for (int rr = 0; rr < kWideRowStep; ++rr)
+        x[q][rr] = (j < cols && r0 + rr < re) ? __ldcs(Z + (size_t)(r0 + rr) * ld + j) : -CUDART_INF_F;
+    }
+#pragma unroll
+    for (int q = 0; q < kWideColsPerThread; ++q) {
+      if (FINAL) {
+#pragma unroll
+        for (int rr = 0; rr < kWideRowStep; ++rr) {           // rows ascending: strict > keeps the first maximum
+          const float t = ((x[q][rr] + urs[rr]) + vj[q]) - d.norm;
+          if (t > a[q]) { a[q] = t; b[q] = __int_as_float(r0 + rr); }
+        }
+      } else {
+#pragma unroll
+        for (int rr = 0; rr < kWideRowStep; ++rr) x[q][rr] += urs[rr];
+        lse_chunk<kWideRowStep>(a[q], b[q], x[q]);
+      }
+    }
+  }
+#pragma unroll
+  for (int q = 0; q < kWideColsPerThread; ++q) {
+    const int j = c0 + q * kWideThreads;
+    if (j < cols) part[(size_t)blockIdx.y * ldp + j] = make_float2(a[q], b[q]);
+  }
+}
+
+// Fixed-order combine of the row-block partials of each column.  FINAL = false: v_j (into v_it, and into v_out after the
+// last iteration).  FINAL = true: column max + first argmax, and the path bit for k_match_finalize.
+template <bool FINAL>
+__global__ void __launch_bounds__(kWideThreads) k_wide_combine(int n0_max, int n1_max, const int* __restrict__ n_dev,
+                                                               const float2* __restrict__ part, size_t ldp,
+                                                               float* __restrict__ v_it, float* __restrict__ v_out,
+                                                               int* __restrict__ idx1, float* __restrict__ max1,
+                                                               unsigned* __restrict__ err) {
+  const WideDims d = wide_dims(n0_max, n1_max, n_dev);
+  const int rows = FINAL ? d.n0 : d.n0 + 1, cols = FINAL ? d.n1 : d.n1 + 1;
+  const int rpb = wide_rows_per_block(rows);
+  const int nb = (rows + rpb - 1) / rpb;
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (FINAL && j == 0) err[kErrPath] = GIMS_STATUS_SINKHORN_WIDE;
+  if (j >= cols) return;
+  float m = -CUDART_INF_F, s = FINAL ? __int_as_float(0x7fffffff) : 0.f;
+  for (int k = 0; k < nb; ++k) {                              // row blocks in order
+    const float2 p = part[(size_t)k * ldp + j];
+    if (FINAL) {
+      if (argmax_better(p.x, __float_as_int(p.y), m, __float_as_int(s))) { m = p.x; s = p.y; }
+    } else {
+      lse_merge_safe(m, s, p.x, p.y);
+    }
+  }
+  if (FINAL) {
+    idx1[j] = __float_as_int(s);
+    max1[j] = m;
+  } else {
+    const float lnu = (j == d.n1) ? d.log_nu_last : d.norm;
+    const float vj = lnu - (m + logf(s));
+    v_it[j] = vj;
+    if (v_out) v_out[j] = vj;
+  }
+}
+
+// iters == 0: the potentials stay 0 (live entries only, as the other kernels leave the rest untouched)
+__global__ void k_wide_zero(int n0_max, int n1_max, const int* __restrict__ n_dev, float* __restrict__ u,
+                            float* __restrict__ v) {
+  const WideDims d = wide_dims(n0_max, n1_max, n_dev);
+  const int t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t <= d.n0) u[t] = 0.f;
+  if (t <= d.n1) v[t] = 0.f;
+}
+
+int launch_wide(const float* Z, int ld, int n0_max, int n1_max, const int* n_dev, int iters, float* u, float* v,
+                float* v_it, float2* part, int* idx0, int* idx1, float* max0, float* max1, unsigned* err, cudaStream_t st) {
+  const size_t ldz = (size_t)ld, ldp = (size_t)n1_max + 1;
+  const unsigned row_grid = (unsigned)cdiv(n0_max + 1, kWideRows);
+  const dim3 col_grid((unsigned)cdiv(n1_max + 1, kWideColsPerThread * kWideThreads), kWideBlocks);
+  const unsigned comb_grid = (unsigned)cdiv(n1_max + 1, kWideThreads);
+  GIMS_CUDA_OK(cudaMemsetAsync(v_it, 0, ldp * sizeof(float), st));
+  if (iters == 0) {
+    k_wide_zero<<<cdiv((n0_max > n1_max ? n0_max : n1_max) + 1, 256), 256, 0, st>>>(n0_max, n1_max, n_dev, u, v);
+    GIMS_LAUNCH_OK();
+  }
+  for (int it = 0; it < iters; ++it) {
+    k_wide_rows<false><<<row_grid, kWideThreads, 0, st>>>(Z, ldz, n0_max, n1_max, n_dev, v_it, u, nullptr, nullptr);
+    GIMS_LAUNCH_OK();
+    k_wide_cols<false><<<col_grid, kWideThreads, 0, st>>>(Z, ldz, n0_max, n1_max, n_dev, u, nullptr, part, ldp);
+    GIMS_LAUNCH_OK();
+    k_wide_combine<false><<<comb_grid, kWideThreads, 0, st>>>(n0_max, n1_max, n_dev, part, ldp, v_it,
+                                                              it == iters - 1 ? v : nullptr, nullptr, nullptr, nullptr);
+    GIMS_LAUNCH_OK();
+  }
+  k_wide_rows<true><<<row_grid, kWideThreads, 0, st>>>(Z, ldz, n0_max, n1_max, n_dev, v_it, u, idx0, max0);
+  GIMS_LAUNCH_OK();
+  k_wide_cols<true><<<col_grid, kWideThreads, 0, st>>>(Z, ldz, n0_max, n1_max, n_dev, u, v_it, part, ldp);
+  GIMS_LAUNCH_OK();
+  k_wide_combine<true><<<comb_grid, kWideThreads, 0, st>>>(n0_max, n1_max, n_dev, part, ldp, nullptr, nullptr, idx1, max1,
+                                                           err);
+  GIMS_LAUNCH_OK();
+  return GIMS_OK;
+}
+
 // Which kernel serves a problem of at most (n0_max + 1) x (n1_max + 1) on a grid of G CTAs — decided on the host from
 // the capacities, so that workspace sizing and launch agree.
 enum SinkKind { kSinkReg = 0, kSinkStream = 1, kSinkExact = 2 };
@@ -1198,8 +1468,12 @@ size_t carve(SinkWs& w, void* base, size_t cap, int n0_max, int n1_max, int grid
 
 // Capacities above which the scaled matrix may need the scratch buffer (the register kernel needs none).  The grid of
 // the launch is not known to the workspace query, so it assumes the streaming kernel whenever the register kernel
-// cannot be guaranteed on a part with >= 128 SMs.
-bool may_stream(int n0_max, int n1_max) { return n0_max + 1 > (kRMax + kRSmem) * 64 || ((n1_max + 1) >> 2) > kThreads; }
+// cannot be guaranteed on a part with >= 128 SMs.  The widest streaming instantiation holds 9 float4 groups per thread
+// (plan()): wider problems never stream, and E ((n0_max + 1) x ld floats, 17.2 GB at 65536 x 65536) is not reserved.
+bool may_stream(int n0_max, int n1_max) {
+  if ((((size_t)n1_max + 1 + 3) >> 2) > (size_t)9 * kThreads) return false;
+  return n0_max + 1 > (kRMax + kRSmem) * 64 || ((n1_max + 1) >> 2) > kThreads;
+}
 
 // Grid of a problem.  The on-chip kernel runs on HALF the SMs whenever its slab then still fits (<= 32 rows per CTA):
 // an iteration is bound by the grid-wide exchange, which gets cheaper with fewer CTAs about as fast as the arithmetic
@@ -1237,12 +1511,15 @@ extern "C" int gims_debug_sinkhorn_trace(long long* dev_buf) {
 
 extern "C" int gims_couplings_ld(int n1_max) { return coup_ld(n1_max); }
 
+// (kMaxGrid rows of partials: the largest grid of the cooperative kernels and the row blocks of the wide path)
 extern "C" size_t gims_sinkhorn_workspace_bytes(int n0_max, int n1_max) {
   SinkWs w;
   return carve(w, nullptr, 0, n0_max, n1_max, kMaxGrid, may_stream(n0_max, n1_max));
 }
 
-// largest n1_max (image-1 keypoints) whose potentials fit the kernels' shared memory, for n0_max <= GIMS_MAX_KPTS
+// largest n1_max (image-1 keypoints) whose potentials fit the scaled-kernel kernels' budget for n0_max <= GIMS_MAX_KPTS,
+// capped at the widest streaming instantiation; the exact kernel serves wider problems while its potentials fit shared
+// memory, the wide path the rest (plan())
 extern "C" int gims_sinkhorn_max_columns(void) {
   int dev = 0, sms = 0, smem_optin = 0;
   if (cudaGetDevice(&dev) != cudaSuccess ||
@@ -1275,18 +1552,28 @@ extern "C" int gims_sinkhorn_match(const float* couplings, int ld, int n0_max, i
   const SinkGrid grid = choose_grid(n0_max, n1_max, sms, smem_optin, iters);
   const int G = grid.G;
   const bool with_e = may_stream(n0_max, n1_max);
-  SinkWs w;
-  size_t need = carve(w, workspace, workspace_bytes, n0_max, n1_max, G, with_e);
-  if (need > workspace_bytes) { set_error("gims_sinkhorn_match: workspace %zu < %zu", workspace_bytes, need); return GIMS_ERR_WORKSPACE; }
   // 128-bit loads of whole rows need a 16-byte aligned base and pitch (gims_couplings_ld gives such a pitch); the scratch
   // matrix E uses the caller's pitch
   const bool vec_ok = with_e && (ld % 4 == 0) && (reinterpret_cast<uintptr_t>(couplings) % 16 == 0) &&
                       (size_t)ld == (((size_t)n1_max + 1 + 3) & ~(size_t)3);
   SinkPlan p;
-  if (!plan(p, n0_max, n1_max, G, smem_optin, vec_ok, iters)) {
-    set_error("gims_sinkhorn_match: n1_max=%d needs more shared memory than an SM has (limit %d columns)", n1_max,
-              gims_sinkhorn_max_columns());
-    return GIMS_ERR_ARG;
+  // potentials wider than the shared memory of the cooperative kernels: the wide path
+  const bool wide = !plan(p, n0_max, n1_max, G, smem_optin, vec_ok, iters);
+  SinkWs w;
+  size_t need = carve(w, workspace, workspace_bytes, n0_max, n1_max, wide ? kMaxGrid : G, with_e);
+  if (need > workspace_bytes) { set_error("gims_sinkhorn_match: workspace %zu < %zu", workspace_bytes, need); return GIMS_ERR_WORKSPACE; }
+  if (wide) {
+    GIMS_CUDA_OK(cudaMemsetAsync(w.err, 0, w.zero_bytes, st));
+    {
+      ProfScope prof(GIMS_PROF_SINKHORN, st);
+      GIMS_TRY(launch_wide(couplings, ld, n0_max, n1_max, n_dev, iters, u, v, w.vg, w.part, indices0, indices1, w.max0,
+                           w.max1, w.err, st));
+    }
+    const int m = n0_max > n1_max ? n0_max : n1_max;
+    k_match_finalize<<<cdiv(m, 256), 256, 0, st>>>(n0_max, n1_max, n_dev, indices0, indices1, w.max0, match_threshold,
+                                                   matches0, matches1, mscores0, mscores1, w.err, status_dev);
+    GIMS_LAUNCH_OK();
+    return GIMS_OK;
   }
   const int budget = smem_optin - 6144;
   SinkArgs a;

@@ -54,8 +54,11 @@ extern "C" {
 #define GIMS_MAX_LAYERS     64
 #define GIMS_MAX_KENC        8
 #define GIMS_MAX_BATCH       4   /* pairs per gims_forward_pairs call */
-#define GIMS_MAX_KPTS    16384   /* per image: the AGC cosine matrix is n^2 fp32 (1 GiB), the Sinkhorn kernel keeps
-                                    2(n+1) floats of potentials in shared memory */
+#define GIMS_MAX_KPTS    65536   /* per image.  Memory does not bound it (the AGC cosine matrix is n^2 fp32 = 16 GiB, the
+                                    couplings (n+1) x ld fp32 = 17.2 GB at this size); the index arithmetic does: element
+                                    offsets into those matrices are 64-bit, the AGC rank select counts the n(n-1)/2 < 2^31
+                                    pairs in 32 bits, and every node id is below 65536, so the component
+                                    search keeps its union-find parents as 16-bit words in shared memory (128 KB) */
 
 /* status word written by the kernels into `gims_pair_outputs.status_dev` / the `status_dev` arguments.
  * Error bits (the host side raises on them): */
@@ -67,6 +70,8 @@ extern "C" {
 /* Information bits: which Sinkhorn iteration the launch ran */
 #define GIMS_STATUS_SINKHORN_FAST   0x100u /* exp-free scaled-kernel iteration */
 #define GIMS_STATUS_SINKHORN_EXACT  0x200u /* log-sum-exp iteration (fallback) */
+#define GIMS_STATUS_SINKHORN_WIDE   0x400u /* log-sum-exp iteration streamed from global memory: problems whose potentials
+                                              do not fit the shared memory of the kernels above */
 
 typedef struct gims_model gims_model;
 
@@ -222,8 +227,13 @@ GIMS_API int gims_final_scores(const gims_model* m, const float* desc, int n0_ma
  *   indices0/1 int32  pre-threshold row/column argmax (gmatcher.py:284-285)
  *   matches0/1 int64 (-1 = unmatched), mscores0/1 fp32 (gmatcher.py:286-294)
  *   status_dev (may be NULL): GIMS_STATUS_SINKHORN_* bits are OR-ed in
- * workspace: gims_sinkhorn_workspace_bytes(n0_max, n1_max).  n1_max is limited by shared memory
- * (gims_sinkhorn_max_columns()). */
+ * workspace: gims_sinkhorn_workspace_bytes(n0_max, n1_max).
+ * gims_sinkhorn_max_columns() is a column count up to which the scaled-kernel kernels are built for every n0_max <=
+ * GIMS_MAX_KPTS: capped at the widest streaming instantiation, 18427 on a B200.  It is not where the WIDE path starts:
+ * the EXACT kernel serves wider problems as long as its potentials fit shared memory (about 56 k columns on a B200).
+ * Problems wider than that run the WIDE path: three non-cooperative launches per iteration (a row pass, per-row-block
+ * column partials, a fixed-order combine of those partials), no float atomics and no grid-wide waits, deterministic run
+ * to run (GIMS_STATUS_SINKHORN_WIDE says it ran). */
 GIMS_API int gims_sinkhorn_max_columns(void);
 GIMS_API size_t gims_sinkhorn_workspace_bytes(int n0_max, int n1_max);
 GIMS_API int gims_sinkhorn_match(const float* couplings, int ld, int n0_max, int n1_max, const int* n_dev, int iters,
